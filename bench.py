@@ -93,9 +93,10 @@ class ClockSampler:
                 "reasons": reasons, "samples": len(sm)}
 
 
-def cuda_time_steps(torch, dist, world, steps, warmup, step_fn, flush_fn):
+def cuda_time_steps(torch, dist, world, steps, warmup, step_fn, flush_fn, before_last=None):
     """W warm-up steps, then K steps each bracketed by CUDA events on the
-    current stream (L2 flush between steps, outside the events); barrier +
+    current stream (L2 flush between steps, outside the events; before_last,
+    if given, runs outside the events ahead of the last step); barrier +
     synchronize on both sides; returns max-over-ranks total ms."""
     for _ in range(warmup):
         step_fn()
@@ -104,7 +105,9 @@ def cuda_time_steps(torch, dist, world, steps, warmup, step_fn, flush_fn):
         dist.barrier()
     torch.cuda.synchronize()
     evs = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(steps)]
-    for a, b in evs:
+    for i, (a, b) in enumerate(evs):
+        if before_last is not None and i == steps - 1:
+            before_last()
         flush_fn()
         a.record()
         step_fn()
@@ -119,6 +122,26 @@ def cuda_time_steps(torch, dist, world, steps, warmup, step_fn, flush_fn):
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
         total = float(t.item())
     return total
+
+
+DUMP_MAX_ELEMS = 1 << 22  # per array: 16 MiB of float32, so the dump of all three workloads stays under 64 MiB
+
+
+def dump_outputs(torch, out_dir, prefix, arrays):
+    """Writes each device array as <out_dir>/<prefix>_<key>.npy in float32.  An array longer than DUMP_MAX_ELEMS is
+    replaced by a fixed sample: one element out of every stretch of n // DUMP_MAX_ELEMS, at an offset drawn from a
+    generator seeded with n, so every run writes the same positions."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for key, t in arrays.items():
+        t = t.detach().reshape(-1).float()
+        n = t.numel()
+        if n > DUMP_MAX_ELEMS:
+            stride = n // DUMP_MAX_ELEMS
+            idx = np.arange(DUMP_MAX_ELEMS, dtype=np.int64) * stride + \
+                np.random.default_rng(n).integers(0, stride, DUMP_MAX_ELEMS)
+            t = t[torch.from_numpy(idx).to(t.device)]
+        np.save(os.path.join(out_dir, f"{prefix}_{key}.npy"), t.cpu().numpy().astype(np.float32))
 
 
 def algorithmic_bytes(P, world, mode, zero_diff, bf16, nvls=False, push=False):
@@ -282,6 +305,7 @@ def measure_workload(torch, dist, C, harness, nets, args, name, grad_dtype, rank
     prod = harness.make_producer(name, net)
     cl.start()
     P = net.param_count()
+    w0 = net.data().clone() if args.dump_outputs else None
     mode = int(net.get_option("resolved_algo"))
     zero = int(net.get_option("zero_diff"))
     kern = int(net.get_option("resolved_kernel"))
@@ -311,6 +335,7 @@ def measure_workload(torch, dist, C, harness, nets, args, name, grad_dtype, rank
 
     # Net::ForwardBackward, captured in a CUDA graph when possible (launch-bound for the small nets)
     graph = None
+    last = {}  # the loss of the latest forward/backward
     if not args.no_graph:
         try:
             side = torch.cuda.Stream()
@@ -322,7 +347,7 @@ def measure_workload(torch, dist, C, harness, nets, args, name, grad_dtype, rank
             torch.cuda.synchronize()
             graph = torch.cuda.CUDAGraph()
             with torch.cuda.graph(graph):
-                prod.forward_backward(x_dev, y_dev)
+                last["loss"] = prod.forward_backward(x_dev, y_dev)
             net.diff().zero_()
         except Exception as e:  # eager fallback for the producer only (not the product path)
             graph = None
@@ -335,7 +360,7 @@ def measure_workload(torch, dist, C, harness, nets, args, name, grad_dtype, rank
         if graph is not None:
             graph.replay()
         else:
-            prod.forward_backward(x_dev, y_dev)
+            last["loss"] = prod.forward_backward(x_dev, y_dev)
 
     def step():
         fb()
@@ -356,11 +381,27 @@ def measure_workload(torch, dist, C, harness, nets, args, name, grad_dtype, rank
         if int(spin.item()) == 0:
             break
     torch.cuda.synchronize()
+
+    def restart():
+        # --dump-outputs: how many steps ran before the last timed one depends on the clock (the loop above), so
+        # that step starts from the initial weights, zero history, iteration 0 and a reseeded dropout generator:
+        # its outputs are then the same from run to run
+        net.data().copy_(w0)
+        net.history().zero_()
+        net.diff().zero_()
+        net.set_option("iter", 0)
+        torch.cuda.manual_seed(1234)
+
     launches0 = net.launch_count()
-    total_ms = cuda_time_steps(torch, dist, world, args.steps, args.warmup, step, flush)
+    total_ms = cuda_time_steps(torch, dist, world, args.steps, args.warmup, step, flush,
+                               before_last=restart if args.dump_outputs else None)
     launches = net.launch_count() - launches0 - args.warmup
     if not net.synchronize():
         raise RuntimeError(net.last_error())
+    if args.dump_outputs and rank == 0:
+        o, n = net.shard() if world > 1 else (0, P)  # history is kept on the owner of each shard
+        dump_outputs(torch, args.dump_outputs, name + ("_bf16" if bf16 else ""),
+                     {"weights": net.data(), "history": net.history()[o:o + n], "loss": last["loss"]})
 
     # The fused kernel IN the step: library-side CUDA events around the one launch, on the launching stream,
     # with forward/backward queued right in front of it (so the ranks arrive as they do in training: skewed by
@@ -940,6 +981,9 @@ def main():
     ap.add_argument("--zero-diff", type=int, default=1, help="sweep: fold ClearParamDiffs into the kernel")
     ap.add_argument("--sweep-min-bytes", type=int, default=0)
     ap.add_argument("--sweep-max-bytes", type=int, default=1 << 40)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the weights, momentum history and loss that the last timed step of each workload "
+                         "computed as DIR/<workload>_<name>.npy (float32; arrays over 4 Mi elements as a fixed sample)")
     args = ap.parse_args()
     args.warmup = max(3, args.warmup)
     if args.impl == "reference" and args.sweep:

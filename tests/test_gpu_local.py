@@ -62,9 +62,10 @@ def test_zero_diff_can_be_disabled(cos, oracle):
         R.close()
 
 
-def test_boundary_conventions_like_CaffeNetTest(cos):
+def test_boundary_conventions_like_CaffeNetTest(cos, tmp_path):
     # CaffeNetTest.java:86-159 on a local net
-    desc = cos.SolverDesc([100, 10], max_iter=2000, snapshot_prefix="/tmp/cos_test_local", **HP_CIFAR)
+    prefix = str(tmp_path / "cos_test_local")
+    desc = cos.SolverDesc([100, 10], max_iter=2000, snapshot_prefix=prefix, **HP_CIFAR)
     net = cos.CaffeNet(desc)
     try:
         assert net.init(-1) is False
@@ -86,7 +87,7 @@ def test_boundary_conventions_like_CaffeNetTest(cos):
         import os
         for is_state in (True, False):
             fn = net.snapshotFilename(it, is_state)
-            assert fn.startswith("/tmp/cos_test_local_iter_0") and os.path.exists(fn)
+            assert fn.startswith(prefix + "_iter_0") and os.path.exists(fn)
             os.unlink(fn)
         with pytest.raises(cos.CosError, match="data is NULL"):  # trainnull
             net.train(0, None)

@@ -2,9 +2,9 @@
 
 There is no libhdf5 / h5py in this environment, so the evidence is layered:
   1. the C++ READER is pinned on files libhdf5 itself wrote -- the reference's fixtures
-     caffe-public/src/caffe/test/test_data/{solver_data,sample_data}.h5 (read where they lie, skipped when the
-     reference tree is absent) -- against (a) the raw bytes at the data offsets and (b) a second, independent
-     mini-parser of the format written in Python below;
+     caffe-public/src/caffe/test/test_data/{solver_data,sample_data}.h5, stored under tests/golden/hdf5 --
+     against (a) the raw bytes at the data offsets and (b) a second, independent mini-parser of the format
+     written in Python below;
   2. the C++ WRITER's files are parsed by that Python mini-parser (not by the C++ reader alone), their message
      bytes are compared with the libhdf5-written ones, and they round-trip through the C++ reader;
   3. what the format cannot express here (chunked / gzip datasets) is rejected with a clear error.
@@ -15,10 +15,8 @@ import os
 import struct
 
 import numpy as np
-import pytest
 
-FIX = "/root/reference/caffe-public/src/caffe/test/test_data"
-needs_ref = pytest.mark.skipif(not os.path.isdir(FIX), reason="reference fixtures not present")
+FIX = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "hdf5")
 
 
 # ------------------------------------------------------------------ independent mini-parser (Python)
@@ -132,7 +130,6 @@ def _read(L, path, dataset):
     return out, list(dims[:nd.value])
 
 
-@needs_ref
 def test_reader_is_pinned_on_libhdf5_written_fixtures(cos):
     from caffeonspark_b200 import _lib
     L = _lib.lib()
@@ -194,16 +191,16 @@ def test_written_model_has_the_structure_libhdf5_writes(cos, tmp_path):
     assert np.array_equal(out, arrays[4].ravel())
     assert L.cos_caffemodel_read(path.encode(), b"conv2", 1, out.ctypes.data, out.size) == 50
     assert L.cos_caffemodel_read(path.encode(), b"nope", 0, None, 0) == -1
-    if os.path.isdir(FIX):  # message bytes identical to what libhdf5 wrote for a float32 dataset
-        ref = MiniH5(os.path.join(FIX, "solver_data.h5")).objects["/data"]["messages"]
-        mine = mini.objects["/data/conv1/0"]["messages"]
-        for t in (0x0003, 0x0005):  # datatype, fill value (flags + body)
-            assert mine[t] == ref[t], hex(t)
-        assert mine[0x0001][1][:8] == ref[0x0001][1][:8]  # dataspace: version 1, rank 4, max dims present
-        assert mine[0x0008][1][:2] == ref[0x0008][1][:2] and mine[0x0008][0] == ref[0x0008][0]  # layout v3 contiguous
-        # same message types (libhdf5 pads its 256-byte header block with a NIL message, type 0)
-        assert sorted(mine) == sorted(t for t in ref if t != 0) == [0x01, 0x03, 0x05, 0x08, 0x12]
-        assert mini.root_cache[0] == 1  # root entry caches B-tree / heap like libhdf5's
+    # message bytes identical to what libhdf5 wrote for a float32 dataset
+    ref = MiniH5(os.path.join(FIX, "solver_data.h5")).objects["/data"]["messages"]
+    mine = mini.objects["/data/conv1/0"]["messages"]
+    for t in (0x0003, 0x0005):  # datatype, fill value (flags + body)
+        assert mine[t] == ref[t], hex(t)
+    assert mine[0x0001][1][:8] == ref[0x0001][1][:8]  # dataspace: version 1, rank 4, max dims present
+    assert mine[0x0008][1][:2] == ref[0x0008][1][:2] and mine[0x0008][0] == ref[0x0008][0]  # layout v3 contiguous
+    # same message types (libhdf5 pads its 256-byte header block with a NIL message, type 0)
+    assert sorted(mine) == sorted(t for t in ref if t != 0) == [0x01, 0x03, 0x05, 0x08, 0x12]
+    assert mini.root_cache[0] == 1  # root entry caches B-tree / heap like libhdf5's
 
 
 def test_solverstate_h5_round_trip_and_many_links(cos, tmp_path):

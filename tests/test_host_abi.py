@@ -4,6 +4,7 @@ every symbol include/caffedistri_b200.h declares, the pure host functions
 reference's config files, and compute entry points FAIL LOUDLY without a GPU.
 No device compute is attempted here."""
 import ctypes
+import json
 import os
 import re
 
@@ -75,27 +76,30 @@ def test_layout_parser_on_generated_prototxt(cos, tmp_path):
         assert d.batch_size == nets.NETS[name]["batch"]
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/data"), reason="reference tree not on this box")
+CONFIGS = os.path.join(ROOT, "tests", "golden", "configs")
+
+
 def test_layout_parser_on_reference_config_files(cos):
-    # SURVEY.md App. D: the reference's own prototxts must yield these layouts
+    # SURVEY.md App. D: the reference's own prototxts (its data/ and caffe-distri/src/test/resources/ files,
+    # stored under tests/golden/configs) must yield these layouts
     want = {"lenet_memory_solver.prototxt": (431080, 8, "inv", 64),
             "cifar10_quick_solver.prototxt": (145578, 10, "fixed", 100),
             "bvlc_reference_solver.prototxt": (60965224, 16, "step", 2),
             "lenet_cos_solver.prototxt": (431080, 8, None, None)}
     for f, (P, nblobs, pol, batch) in want.items():
-        d = cos.parse_solver("/root/reference/data/" + f)
+        d = cos.parse_solver(os.path.join(CONFIGS, "data", f))
         assert d.param_count == P and len(d.counts) == nblobs
         if pol:
             assert d.lr_policy == pol and d.batch_size == batch
-    d = cos.parse_solver("/root/reference/data/bvlc_reference_solver.prototxt")
+    d = cos.parse_solver(os.path.join(CONFIGS, "data", "bvlc_reference_solver.prototxt"))
     assert d.decay_mult[1::2] == [0.0] * 8 and d.lr_mult[1::2] == [2.0] * 8  # biases: lr 2, decay 0
     # every other CaffeOnSpark configuration on the path: DataFrame-fed LeNet and the JNI test's CaffeNet
     # (fc8 with 2 outputs: 60,965,224 - (4,096,000 + 1000) + (4096 * 2 + 2))
-    assert cos.parse_solver("/root/reference/data/lenet_dataframe_solver.prototxt").param_count == 431080
-    t = cos.parse_solver("/root/reference/caffe-distri/src/test/resources/caffenet_solver.prototxt")
+    assert cos.parse_solver(os.path.join(CONFIGS, "data", "lenet_dataframe_solver.prototxt")).param_count == 431080
+    t = cos.parse_solver(os.path.join(CONFIGS, "test_resources", "caffenet_solver.prototxt"))
     assert t.param_count == 60965224 - 4097000 + 8194 == 56876418 and t.batch_size == 4
     with pytest.raises(cos.CosError, match="clip_gradients"):  # LRCN: clipping + LSTM are off the accelerated path
-        cos.parse_solver("/root/reference/data/lrcn_solver.prototxt")
+        cos.parse_solver(os.path.join(CONFIGS, "data", "lrcn_solver.prototxt"))
 
 
 def test_parser_rejects_what_is_off_the_path(cos, tmp_path):
@@ -169,9 +173,10 @@ def test_adapter_loopback_two_ranks_in_process(cos):
 
 
 def test_jni_shim_type_checks_and_covers_the_18_natives():
-    """No JDK here: the JNI shim is type-checked against a stand-in jni.h and
+    """Without a JDK, the JNI shim is type-checked against a stand-in jni.h and
     must define one Java_com_yahoo_ml_jcaffe_CaffeNet_* export per native the
-    reference's CaffeNet.java declares (CaffeNet.java:60-230)."""
+    reference's CaffeNet.java declares (CaffeNet.java:60-230; the list is stored
+    in tests/golden/reference_interfaces.json)."""
     import subprocess
     src = os.path.join(ROOT, "caffeonspark_b200", "csrc", "jni_shim.cpp")
     r = subprocess.run(["g++", "-std=c++17", "-fsyntax-only", "-Wall", "-Werror", "-I",
@@ -183,10 +188,9 @@ def test_jni_shim_type_checks_and_covers_the_18_natives():
     text = open(src).read()
     for n in natives:
         assert f"Java_com_yahoo_ml_jcaffe_CaffeNet_{n}(" in text, n
-    if os.path.isdir("/root/reference"):
-        java = open("/root/reference/caffe-distri/src/main/java/com/yahoo/ml/jcaffe/CaffeNet.java").read()
-        declared = set(re.findall(r"native\s+[\w\[\]]+\s+(\w+)\s*\(", java))
-        assert declared == set(natives), declared ^ set(natives)
+    with open(os.path.join(ROOT, "tests", "golden", "reference_interfaces.json")) as f:
+        declared = set(json.load(f)["caffenet_java_natives"])
+    assert declared == set(natives), declared ^ set(natives)
 
 
 def test_every_entry_point_survives_null_and_invalid_arguments(cos):
@@ -361,15 +365,27 @@ def test_bench_algorithmic_byte_model_matches_design():
     assert spec is not None
 
 
-def test_adapter_pathname_sockets_for_separate_containers(cos, tmp_path, monkeypatch):
+@pytest.fixture
+def sock_dir():
+    """A fresh directory with a short path: a socket path must fit sun_path (108 bytes), which pytest's tmp_path
+    under a deep $TMPDIR does not."""
+    import pathlib
+    import shutil
+    import tempfile
+    d = tempfile.mkdtemp(prefix="cos", dir="/tmp")
+    yield pathlib.Path(d)
+    shutil.rmtree(d, ignore_errors=True)
+
+
+def test_adapter_pathname_sockets_for_separate_containers(cos, sock_dir, monkeypatch):
     """COS_SOCKET_DIR: endpoints become socket files in a shared directory (executors that do not share a network
     namespace cannot see each other's abstract sockets); same protocol, files removed on close."""
     import threading
-    monkeypatch.setenv("COS_SOCKET_DIR", str(tmp_path))
+    monkeypatch.setenv("COS_SOCKET_DIR", str(sock_dir))
     ads = [cos.PeerAdapter(2, r) for r in range(2)]
     addrs = [a.address() for a in ads]
-    assert all(a.startswith("cosb200://") and str(tmp_path) in a and a.endswith(".sock") for a in addrs)
-    assert len(list(tmp_path.glob("*.sock"))) == 2
+    assert all(a.startswith("cosb200://") and str(sock_dir) in a and a.endswith(".sock") for a in addrs)
+    assert len(list(sock_dir.glob("*.sock"))) == 2
     oks = [None, None]
     th = [threading.Thread(target=lambda r=r: oks.__setitem__(r, ads[r].connect(addrs) and ads[r].barrier(5000)))
           for r in range(2)]
@@ -385,9 +401,9 @@ def test_adapter_pathname_sockets_for_separate_containers(cos, tmp_path, monkeyp
     os.close(got)
     os.close(fd)
     [a.close() for a in ads]
-    assert list(tmp_path.glob("*.sock")) == []
+    assert list(sock_dir.glob("*.sock")) == []
     monkeypatch.delenv("COS_SOCKET_DIR")
     a = cos.PeerAdapter(2, 0)
-    assert not a.connect(["", "cosb200://1/" + str(tmp_path) + "/cosb200-1-r1-00.sock"])  # nobody there
+    assert not a.connect(["", "cosb200://1/" + str(sock_dir) + "/cosb200-1-r1-00.sock"])  # nobody there
     assert not a.connect(["", "cosb200://1//etc/passwd"])                                   # not one of ours
     a.close()
