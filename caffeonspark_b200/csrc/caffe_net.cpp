@@ -321,7 +321,6 @@ bool CaffeNet::launch(int mode, cudaStream_t stream, std::string* err) {
   p.ll_weight_stride = ll_weight_stride_;
   p.nvls_unroll = opt_nvls_unroll_;
   p.nvls_p2p = opt_nvls_p2p_;
-  p.use_nvls = nvls_active_ ? 1 : 0;
   p.mc_data = nvls_active_ ? reinterpret_cast<float*>(mc_base_ + off_data_) : nullptr;
   p.mc_diff = nvls_active_ ? reinterpret_cast<const float*>(mc_base_ + off_diff_) : nullptr;
   p.hist = hist_;

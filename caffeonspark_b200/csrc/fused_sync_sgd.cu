@@ -77,11 +77,10 @@ template <bool BF16>
 __device__ __forceinline__ float reduce_scalar(const SyncParams& p, int s, uint64_t i) {
   float acc = 0.f;
   for (int j = 0; j < p.world; ++j) {
-    int src = s + j;
-    if (src >= p.world) src -= p.world;
-    float x = BF16 ? bf16_bits_to_float(p.wire[src][i]) : p.diff[src][i];
-    x = __fmul_rn(p.inv_scale, x);
-    acc = (j == 0) ? x : __fadd_rn(x, acc);
+    const int src = peer(s, j, p.world);
+    const float x = BF16 ? bf16_bits_to_float(p.wire[src][i]) : p.diff[src][i];
+    if (j == 0) acc = scaled(p.inv_scale, x);
+    else add_scaled(acc, p.inv_scale, x);
   }
   return acc;
 }
@@ -138,17 +137,11 @@ __global__ void __launch_bounds__(kDefaultThreads, 2) fused_sync_sgd_kernel(cons
       const ShardRange r = shard_range(p.count, world, s);
       for (uint64_t j = tid; j < r.nvec; j += stride) {
         const uint64_t i = (r.vec_lo + j) << 2;
-        float4 v = ld_stream(g + i);
-        uint2 o;
-        o.x = static_cast<uint32_t>(float_to_bf16_bits(v.x)) | (static_cast<uint32_t>(float_to_bf16_bits(v.y)) << 16);
-        o.y = static_cast<uint32_t>(float_to_bf16_bits(v.z)) | (static_cast<uint32_t>(float_to_bf16_bits(v.w)) << 16);
-        *reinterpret_cast<uint2*>(wv + i) = o;
+        *reinterpret_cast<uint2*>(wv + i) = pack_bf16x4(ld_stream(g + i));
       }
       if (blockIdx.x == 0) {
-        const uint64_t nhead = r.head_end - r.lo, ntail = r.hi - r.tail_begin;
-        if (threadIdx.x < nhead) wv[r.lo + threadIdx.x] = float_to_bf16_bits(g[r.lo + threadIdx.x]);
-        else if (threadIdx.x - nhead < ntail)
-          wv[r.tail_begin + (threadIdx.x - nhead)] = float_to_bf16_bits(g[r.tail_begin + (threadIdx.x - nhead)]);
+        const uint64_t i = edge_element(r, threadIdx.x);
+        if (i != ~0ull) wv[i] = float_to_bf16_bits(g[i]);
       }
     }
   }
@@ -210,56 +203,22 @@ __global__ void __launch_bounds__(kDefaultThreads, 2) fused_sync_sgd_kernel(cons
         float4 g;
         if (p.mode == kModeLocal) {
           g = ld_stream(p.diff[rank] + i);  // no scale at N == 1 (CaffeNet.cpp:206-216: no sync object)
-          if (BF16) {  // bf16 gradient inputs: same rounding the wire applies at N > 1
-            g.x = bf16_bits_to_float(float_to_bf16_bits(g.x));
-            g.y = bf16_bits_to_float(float_to_bf16_bits(g.y));
-            g.z = bf16_bits_to_float(float_to_bf16_bits(g.z));
-            g.w = bf16_bits_to_float(float_to_bf16_bits(g.w));
-          }
+          if (BF16) g = round_bf16x4(g);  // bf16 gradient inputs: same rounding the wire applies at N > 1
         } else {
           g = reduce_vec_any<N, BF16>(p, s, i);
         }
         sgd_vec(p, cur, i, g, w, h);
         *reinterpret_cast<float4*>(hl + i) = h;
         *reinterpret_cast<float4*>(wl + i) = w;
-        if (push) {
-#pragma unroll
-          for (int q = 1; q < (N > 0 ? N : 1); ++q) {
-            int dst = rank + q;
-            if (dst >= world) dst -= world;
-            st_vec(p.data[dst] + i, w);
-          }
-          if (N == 0) {
-            for (int q = 1; q < world; ++q) {
-              int dst = rank + q;
-              if (dst >= world) dst -= world;
-              st_vec(p.data[dst] + i, w);
-            }
-          }
-        }
+        if (push) for_peers<N>(world, [&](int q) { st_vec(p.data[peer(rank, q, world)] + i, w); });
       }
       if (blockIdx.x == 0) {  // scalar head / tail of the range (<= 3 elements each)
-        const uint64_t nhead = r.head_end - r.lo, ntail = r.hi - r.tail_begin;
-        uint64_t i = ~0ull;
-        if (threadIdx.x < nhead) i = r.lo + threadIdx.x;
-        else if (threadIdx.x - nhead < ntail) i = r.tail_begin + (threadIdx.x - nhead);
+        const uint64_t i = edge_element(r, threadIdx.x);
         if (i != ~0ull) {
-          SegCursor c2 = cur;
-          c2.seek(i);
           float g = (p.mode == kModeLocal) ? p.diff[rank][i] : reduce_scalar<BF16>(p, s, i);
-          if (BF16 && p.mode == kModeLocal) g = bf16_bits_to_float(float_to_bf16_bits(g));
-          float w = wl[i], h = hl[i];
-          sgd_element(g, w, h, __fmul_rn(p.rate, c2.lr_mult[c2.k]), __fmul_rn(p.weight_decay, c2.decay_mult[c2.k]),
-                      p.momentum, p.l1);
-          hl[i] = h;
-          wl[i] = w;
-          if (push) {
-            for (int q = 1; q < world; ++q) {
-              int dst = rank + q;
-              if (dst >= world) dst -= world;
-              p.data[dst][i] = w;
-            }
-          }
+          if (BF16 && p.mode == kModeLocal) g = round_bf16(g);
+          const float w = sgd_scalar(p, cur, i, g, wl, hl);
+          if (push) store_peers(p, world, i, w);
         }
       }
     }
@@ -284,11 +243,7 @@ __global__ void __launch_bounds__(kDefaultThreads, 2) fused_sync_sgd_kernel(cons
       for (int s = 0; s < world; ++s) {
         const ShardRange r = shard_range(p.count, world, s);
         for (uint64_t j = tid; j < r.nvec; j += stride) *reinterpret_cast<float4*>(g + ((r.vec_lo + j) << 2)) = z;
-        if (blockIdx.x == 0) {
-          const uint64_t nhead = r.head_end - r.lo, ntail = r.hi - r.tail_begin;
-          if (threadIdx.x < nhead) g[r.lo + threadIdx.x] = 0.f;
-          else if (threadIdx.x - nhead < ntail) g[r.tail_begin + (threadIdx.x - nhead)] = 0.f;
-        }
+        zero_edges(g, r);
       }
     }
   }
@@ -316,33 +271,17 @@ uint64_t host_mix64(uint64_t z) {
   return z ^ (z >> 31);
 }
 
-template <int N>
-cudaError_t launch_n(const SyncParams& p, int grid, int block, size_t smem, cudaStream_t stream) {
-  if (p.grad_bf16) fused_sync_sgd_kernel<N, true><<<grid, block, smem, stream>>>(p);
-  else fused_sync_sgd_kernel<N, false><<<grid, block, smem, stream>>>(p);
-  return cudaGetLastError();
-}
-
 }  // namespace
 
 int default_sync_grid(int device) {
-  int sms = 0;
-  if (cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device) != cudaSuccess || sms <= 0) {
-    cudaGetLastError();
-    sms = 148;
-  }
-  return 2 * sms;  // __launch_bounds__(512, 2): two resident CTAs per SM
+  return 2 * sm_count(device);  // __launch_bounds__(512, 2): two resident CTAs per SM
 }
 
 cudaError_t launch_fused_sync_sgd(const SyncParams& p, int grid, int block, cudaStream_t stream) {
-  if (p.world < 1 || p.world > kMaxRanks || p.rank < 0 || p.rank >= p.world) return cudaErrorInvalidValue;
+  if (!check_world(p, 1)) return cudaErrorInvalidValue;
   if (block <= 0) block = kDefaultThreads;
   if (block > kDefaultThreads || block < kMaxRanks || (block & 31)) return cudaErrorInvalidValue;
-  if (grid <= 0) {
-    int dev = 0;
-    cudaGetDevice(&dev);
-    grid = default_sync_grid(dev);
-  }
+  if (grid <= 0) grid = default_sync_grid(-1);
   if (grid > kMaxCtas) grid = kMaxCtas;
   // do not launch more CTAs than there is work for (tiny nets): one vector per thread
   uint64_t work_vecs = (p.mode == kModeOneShot || p.mode == kModeLocal) ? (p.count >> 2)
@@ -351,18 +290,13 @@ cudaError_t launch_fused_sync_sgd(const SyncParams& p, int grid, int block, cuda
   uint64_t need = (work_vecs + block - 1) / block;
   if (need < 1) need = 1;
   if (static_cast<uint64_t>(grid) > need) grid = static_cast<int>(need);
-  size_t smem = p.nseg <= kMaxSegSmem ? static_cast<size_t>(p.nseg) * (sizeof(uint64_t) + 2 * sizeof(float)) : 0;
+  const size_t smem = seg_smem_bytes(p, kMaxSegSmem);
   const int n = (p.mode == kModeLocal || p.mode == kModeAllGather) ? 0 : p.world;
-  switch (n) {
-    case 2: return launch_n<2>(p, grid, block, smem, stream);
-    case 3: return launch_n<3>(p, grid, block, smem, stream);
-    case 4: return launch_n<4>(p, grid, block, smem, stream);
-    case 5: return launch_n<5>(p, grid, block, smem, stream);
-    case 6: return launch_n<6>(p, grid, block, smem, stream);
-    case 7: return launch_n<7>(p, grid, block, smem, stream);
-    case 8: return launch_n<8>(p, grid, block, smem, stream);
-    default: return launch_n<0>(p, grid, block, smem, stream);
-  }
+  return dispatch_world(n, [&](auto N) {
+    if (p.grad_bf16) fused_sync_sgd_kernel<N, true><<<grid, block, smem, stream>>>(p);
+    else fused_sync_sgd_kernel<N, false><<<grid, block, smem, stream>>>(p);
+    return cudaGetLastError();
+  });
 }
 
 // TMA (cp.async.bulk) pipelined variant: see fused_sync_sgd_tma.cu.

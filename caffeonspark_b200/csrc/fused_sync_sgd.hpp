@@ -47,7 +47,6 @@ struct SyncParams {
   uint64_t ll_weight_stride;        // words per LL weight slot
   float* mc_data;                   // NVLS: multicast address of data_ (a store lands on every rank)
   const float* mc_diff;             // NVLS: multicast address of diff_ (a load returns the in-switch sum)
-  int use_nvls;                     // two-shot only: multimem.ld_reduce / multimem.st instead of P2P
   int nvls_unroll;                  // NVLS kernel: switch loads in flight per thread (1, 2, 4, 8)
   int nvls_p2p;                     // NVLS kernel: of every (nvls_unroll + nvls_p2p) vectors this many go over plain P2P
   float* hist;                      // local SGD history (momentum buffer)
@@ -85,7 +84,7 @@ void ll_slot_words(uint64_t count, int world, bool bf16, uint64_t* grad_words, u
 constexpr uint64_t kLLRegionMaxBytes = 8ull << 20;
 // Elements per receive slot of the push kernel for (count, world).
 uint64_t push_recv_stride(uint64_t count, int world);
-// Occupancy-derived default grid (co-resident CTAs) for the vector kernel.
+// Occupancy-derived default grid (co-resident CTAs) for the vector kernel; device < 0: the current device.
 int default_sync_grid(int device);
 // Device-side synthetic fill, identical to cos_oracle_fill (tests/bench).
 cudaError_t launch_fill(float* out, uint64_t n, uint64_t seed, uint64_t stream_id, float amp,

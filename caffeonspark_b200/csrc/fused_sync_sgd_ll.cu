@@ -124,12 +124,6 @@ __device__ __forceinline__ bool poll1(const uint64_t* w, uint32_t flag, Poll& po
 __device__ __forceinline__ uint64_t edge_index(const ShardRange& r, uint64_t e) {
   return e < r.head_end ? e - r.lo : 4 + (e - r.tail_begin);
 }
-__device__ __forceinline__ uint64_t edge_of_thread(const ShardRange& r, unsigned t) {
-  const uint64_t nhead = r.head_end - r.lo, ntail = r.hi - r.tail_begin;
-  if (t < nhead) return r.lo + t;
-  if (t - nhead < ntail) return r.tail_begin + (t - nhead);
-  return ~0ull;
-}
 
 // N = compile-time world size, 2..8 (the N-1 polled slots live in registers)
 template <int N, bool BF16>
@@ -161,7 +155,6 @@ __global__ void __launch_bounds__(kLLThreads, 1) fused_sync_sgd_ll_kernel(const 
   const uint64_t wslot = p.ll_weight_stride; // 8-byte words per weight slot
   float* g = const_cast<float*>(p.diff[rank]);
   const bool zero = p.zero_diff != 0;
-  const float4 z4 = make_float4(0.f, 0.f, 0.f, 0.f);
   // body word index of element i in a slot of shard range r: fp32 wire / weights 1 element per word,
   // bf16 wire 2 elements per word; base = r.lo rounded down to a multiple of 4
   const uint64_t gedge = gslot - kEdgeWords, wedge = wslot - kEdgeWords;
@@ -205,7 +198,7 @@ __global__ void __launch_bounds__(kLLThreads, 1) fused_sync_sgd_ll_kernel(const 
       int q = rank + d;
       if (q >= world) q -= world;
       const ShardRange r = shard_range(p.count, world, q);
-      const uint64_t e = edge_of_thread(r, threadIdx.x);
+      const uint64_t e = edge_element(r, threadIdx.x);
       if (e != ~0ull) {
         float x = g[e];
         if (BF16) x = bf16_bits_to_float(float_to_bf16_bits(x));
@@ -215,16 +208,7 @@ __global__ void __launch_bounds__(kLLThreads, 1) fused_sync_sgd_ll_kernel(const 
   }
   if (tracer) p.trace[1] = globaltimer_ns();
   if (zero) {  // ClearParamDiffs of what I pushed: plain streaming stores behind the pushes, hidden in the flight time
-    for (int d = 1; d < world; ++d) {
-      int q = rank + d;
-      if (q >= world) q -= world;
-      const ShardRange r = shard_range(p.count, world, q);
-      for (uint64_t j = tid; j < r.nvec; j += stride) st_vec(g + ((r.vec_lo + j) << 2), z4);
-      if (blockIdx.x == 0) {
-        const uint64_t e = edge_of_thread(r, threadIdx.x);
-        if (e != ~0ull) g[e] = 0.f;
-      }
-    }
+    for (int d = 1; d < world; ++d) zero_range<false>(g, shard_range(p.count, world, peer(rank, d, world)), tid, stride);
   }
   if (tracer) p.trace[2] = globaltimer_ns();
 
@@ -300,7 +284,7 @@ __global__ void __launch_bounds__(kLLThreads, 1) fused_sync_sgd_ll_kernel(const 
       }
     }
     if (alive && blockIdx.x == 0) {  // scalar head / tail of my shard
-      const uint64_t e = edge_of_thread(r, threadIdx.x);
+      const uint64_t e = edge_element(r, threadIdx.x);
       if (e != ~0ull) {
         SegCursor c2 = cur;
         c2.seek(e);
@@ -330,11 +314,7 @@ __global__ void __launch_bounds__(kLLThreads, 1) fused_sync_sgd_ll_kernel(const 
       }
     }
     if (zero) {  // my own shard of diff_ (read above by exactly these threads)
-      for (uint64_t j = tid; j < r.nvec; j += stride) st_vec(g + ((r.vec_lo + j) << 2), z4);
-      if (blockIdx.x == 0) {
-        const uint64_t e = edge_of_thread(r, threadIdx.x);
-        if (e != ~0ull) g[e] = 0.f;
-      }
+      zero_range<false>(g, r, tid, stride);
     }
   }
   if (tracer) p.trace[3] = globaltimer_ns();
@@ -374,7 +354,7 @@ __global__ void __launch_bounds__(kLLThreads, 1) fused_sync_sgd_ll_kernel(const 
         int q = rank + d;
         if (q >= world) q -= world;
         const ShardRange r = shard_range(p.count, world, q);
-        const uint64_t e = edge_of_thread(r, threadIdx.x);
+        const uint64_t e = edge_element(r, threadIdx.x);
         if (e != ~0ull) {
           uint32_t u;
           alive = poll1(p.ll_weight[rank] + static_cast<uint64_t>(q) * wslot + wedge + edge_index(r, e), flag, poll, q, u);
@@ -384,13 +364,6 @@ __global__ void __launch_bounds__(kLLThreads, 1) fused_sync_sgd_ll_kernel(const 
     }
   }
   if (tracer) p.trace[4] = globaltimer_ns();
-}
-
-template <int N>
-cudaError_t launch_ll_n(const SyncParams& p, int grid, int block, size_t smem, cudaStream_t stream) {
-  if (p.grad_bf16) fused_sync_sgd_ll_kernel<N, true><<<grid, block, smem, stream>>>(p);
-  else fused_sync_sgd_ll_kernel<N, false><<<grid, block, smem, stream>>>(p);
-  return cudaGetLastError();
 }
 
 }  // namespace
@@ -406,16 +379,14 @@ void ll_slot_words(uint64_t count, int world, bool bf16, uint64_t* grad_words, u
 
 cudaError_t launch_fused_sync_sgd_ll(const SyncParams& p, int grid, int block, int vecs_per_thread,
                                      cudaStream_t stream) {
-  if (p.world < 2 || p.world > kMaxRanks || p.rank < 0 || p.rank >= p.world) return cudaErrorInvalidValue;
+  if (!check_world(p, 2)) return cudaErrorInvalidValue;
   if (p.mode != kModeTwoShot || p.ll_grad_stride == 0 || p.ll_weight_stride == 0) return cudaErrorInvalidValue;
   if (block <= 0) block = kLLThreads;
   if (block > kLLThreads || block < kMaxRanks || (block & 31)) return cudaErrorInvalidValue;
   if (vecs_per_thread <= 0) vecs_per_thread = 2;
   // Every CTA spins on peer data in phases 2 and 3 after feeding the peers in phase 1: the whole grid must be
   // co-resident (__launch_bounds__(512, 1): one CTA per SM).
-  int dev = 0, sms = 148;
-  cudaGetDevice(&dev);
-  cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+  const int sms = sm_count(-1);
   const int cap = sms < kMaxCtas ? sms : kMaxCtas;
   if (grid <= 0) {  // sized by the larger phases (1 and 3 move (N-1)/N of the buffer)
     const uint64_t vecs = (p.count - p.count / p.world) >> 2;
@@ -425,17 +396,16 @@ cudaError_t launch_fused_sync_sgd_ll(const SyncParams& p, int grid, int block, i
     grid = static_cast<int>(need > static_cast<uint64_t>(cap) ? cap : need);
   }
   if (grid > cap) grid = cap;
-  const size_t smem = p.nseg <= kLLMaxSeg ? static_cast<size_t>(p.nseg) * (sizeof(uint64_t) + 2 * sizeof(float)) : 0;
-  switch (p.world) {
-    case 2: return launch_ll_n<2>(p, grid, block, smem, stream);
-    case 3: return launch_ll_n<3>(p, grid, block, smem, stream);
-    case 4: return launch_ll_n<4>(p, grid, block, smem, stream);
-    case 5: return launch_ll_n<5>(p, grid, block, smem, stream);
-    case 6: return launch_ll_n<6>(p, grid, block, smem, stream);
-    case 7: return launch_ll_n<7>(p, grid, block, smem, stream);
-    case 8: return launch_ll_n<8>(p, grid, block, smem, stream);
-    default: return cudaErrorInvalidValue;  // world sizes 9..16 use the barrier-based kernels
-  }
+  const size_t smem = seg_smem_bytes(p, kLLMaxSeg);
+  return dispatch_world(p.world, [&](auto N) {
+    if constexpr (decltype(N)::value == 0) {
+      return cudaErrorInvalidValue;  // world sizes 9..16 use the barrier-based kernels
+    } else {
+      if (p.grad_bf16) fused_sync_sgd_ll_kernel<N, true><<<grid, block, smem, stream>>>(p);
+      else fused_sync_sgd_ll_kernel<N, false><<<grid, block, smem, stream>>>(p);
+      return cudaGetLastError();
+    }
+  });
 }
 
 }  // namespace cosb

@@ -51,17 +51,7 @@ template <int UN, int UP, int N>
 __global__ void __launch_bounds__(kNvlsThreads, 1) fused_sync_sgd_nvls_kernel(const SyncParams p) {
   extern __shared__ unsigned char smem_raw[];
   __shared__ int s_abort;
-  uint64_t* s_end = reinterpret_cast<uint64_t*>(smem_raw);
-  float* s_lr = reinterpret_cast<float*>(s_end + p.nseg);
-  float* s_dm = s_lr + p.nseg;
-  const bool seg_in_smem = p.nseg <= kNvlsMaxSeg;
-  if (seg_in_smem) {
-    for (int k = threadIdx.x; k < p.nseg; k += blockDim.x) {
-      s_end[k] = p.seg_end[k];
-      s_lr[k] = p.seg_lr_mult[k];
-      s_dm[k] = p.seg_decay_mult[k];
-    }
-  }
+  SegCursor cur = load_seg_table(p, smem_raw, kNvlsMaxSeg);
   if (threadIdx.x == 0) s_abort = 0;
   const bool tracer = p.trace != nullptr && blockIdx.x == 0 && threadIdx.x == 0;
   if (tracer) p.trace[0] = globaltimer_ns();
@@ -79,12 +69,6 @@ __global__ void __launch_bounds__(kNvlsThreads, 1) fused_sync_sgd_nvls_kernel(co
 
   if (threadIdx.x < kWorkThreads) {
     // =================== warps 0..14: reduce + update + broadcast ===================
-    SegCursor cur;
-    cur.end = seg_in_smem ? s_end : p.seg_end;
-    cur.lr_mult = seg_in_smem ? s_lr : p.seg_lr_mult;
-    cur.decay_mult = seg_in_smem ? s_dm : p.seg_decay_mult;
-    cur.nseg = p.nseg;
-    cur.k = 0;
     const ShardRange r = shard_range(p.count, world, rank);
     float* wl = p.data[rank];
     float* hl = p.hist;
@@ -108,11 +92,7 @@ __global__ void __launch_bounds__(kNvlsThreads, 1) fused_sync_sgd_nvls_kernel(co
         const uint64_t i = vec_elem(r, j0 + static_cast<uint64_t>(UN + u) * stride);
         if (i != ~0ull) {
 #pragma unroll
-          for (int k = 0; k < NP; ++k) {
-            int src = rank + k;
-            if (src >= NP) src -= NP;
-            x[u][k] = ld_stream(p.diff[src] + i);
-          }
+          for (int k = 0; k < NP; ++k) x[u][k] = ld_stream(p.diff[peer(rank, k, NP)] + i);
         }
       }
 #pragma unroll
@@ -130,19 +110,12 @@ __global__ void __launch_bounds__(kNvlsThreads, 1) fused_sync_sgd_nvls_kernel(co
         if (i != ~0ull) {
           float4 g;
           if (u < UN) {  // in-switch sum over all ranks, then the 1/N scale
-            g = make_float4(__fmul_rn(inv, s[u].x), __fmul_rn(inv, s[u].y), __fmul_rn(inv, s[u].z),
-                            __fmul_rn(inv, s[u].w));
+            g = scaled(inv, s[u]);
           } else {       // reference order: scale first, then r, r+1, ... (mod N)
             const int q = u - UN;
-            g = make_float4(__fmul_rn(inv, x[q][0].x), __fmul_rn(inv, x[q][0].y), __fmul_rn(inv, x[q][0].z),
-                            __fmul_rn(inv, x[q][0].w));
+            g = scaled(inv, x[q][0]);
 #pragma unroll
-            for (int k = 1; k < NP; ++k) {
-              g.x = __fadd_rn(__fmul_rn(inv, x[q][k].x), g.x);
-              g.y = __fadd_rn(__fmul_rn(inv, x[q][k].y), g.y);
-              g.z = __fadd_rn(__fmul_rn(inv, x[q][k].z), g.z);
-              g.w = __fadd_rn(__fmul_rn(inv, x[q][k].w), g.w);
-            }
+            for (int k = 1; k < NP; ++k) add_scaled(g, inv, x[q][k]);
           }
           cur.seek(i);
           sgd_vec(p, cur, i, g, w[u], h[u]);
@@ -152,11 +125,7 @@ __global__ void __launch_bounds__(kNvlsThreads, 1) fused_sync_sgd_nvls_kernel(co
           } else {
             st_vec(wl + i, w[u]);
 #pragma unroll
-            for (int k = 1; k < NP; ++k) {
-              int dst = rank + k;
-              if (dst >= NP) dst -= NP;
-              st_vec(p.data[dst] + i, w[u]);
-            }
+            for (int k = 1; k < NP; ++k) st_vec(p.data[peer(rank, k, NP)] + i, w[u]);
           }
         }
       }
@@ -252,12 +221,7 @@ __global__ void __launch_bounds__(kNvlsThreads, 1) fused_sync_sgd_nvls_kernel(co
   // owners: zero them after barrier B
   if (p.zero_diff && blockIdx.x == 0) {
     float* g = const_cast<float*>(p.diff[rank]);
-    for (int s = 0; s < world; ++s) {
-      const ShardRange q = shard_range(p.count, world, s);
-      const uint64_t nhead = q.head_end - q.lo, ntail = q.hi - q.tail_begin;
-      if (threadIdx.x < nhead) g[q.lo + threadIdx.x] = 0.f;
-      else if (threadIdx.x - nhead < ntail) g[q.tail_begin + (threadIdx.x - nhead)] = 0.f;
-    }
+    for (int s = 0; s < world; ++s) zero_edges(g, shard_range(p.count, world, s));
   }
   if (tracer) p.trace[4] = globaltimer_ns();
 }
@@ -281,17 +245,14 @@ cudaError_t launch_share(const SyncParams& p, int grid, size_t smem, cudaStream_
 }  // namespace
 
 cudaError_t launch_fused_sync_sgd_nvls(const SyncParams& p, int grid, cudaStream_t stream) {
-  if (p.world < 2 || p.world > kMaxRanks || p.rank < 0 || p.rank >= p.world) return cudaErrorInvalidValue;
+  if (!check_world(p, 2)) return cudaErrorInvalidValue;
   if (p.mode != kModeTwoShot || p.grad_bf16 || !p.mc_data || !p.mc_diff) return cudaErrorInvalidValue;
-  int dev = 0, sms = 148;
-  cudaGetDevice(&dev);
-  cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-  if (grid <= 0) grid = sms;  // __launch_bounds__(512, 1): one resident CTA per SM
+  if (grid <= 0) grid = sm_count(-1);  // __launch_bounds__(512, 1): one resident CTA per SM
   if (grid > kMaxCtas) grid = kMaxCtas;
   uint64_t need = (((p.count / p.world) >> 2) + kWorkThreads - 1) / kWorkThreads;  // one vector per work thread
   if (need < 1) need = 1;
   if (static_cast<uint64_t>(grid) > need) grid = static_cast<int>(need);
-  const size_t smem = p.nseg <= kNvlsMaxSeg ? static_cast<size_t>(p.nseg) * (sizeof(uint64_t) + 2 * sizeof(float)) : 0;
+  const size_t smem = seg_smem_bytes(p, kNvlsMaxSeg);
   {  // the per-CTA progress counter has kIterBits bits
     const uint64_t u = static_cast<uint64_t>((p.nvls_unroll > 0 ? p.nvls_unroll : 1) + (p.nvls_p2p > 0 ? 1 : 0));
     const uint64_t per_round = static_cast<uint64_t>(grid) * kWorkThreads * u;

@@ -42,28 +42,6 @@ namespace {
 constexpr int kPushThreads = 512;
 constexpr int kPushMaxSeg = 1024;
 
-__device__ __forceinline__ float round_bf16(float x) { return bf16_bits_to_float(float_to_bf16_bits(x)); }
-
-__device__ __forceinline__ uint2 pack_bf16x4(const float4& v) {
-  uint2 o;
-  o.x = static_cast<uint32_t>(float_to_bf16_bits(v.x)) | (static_cast<uint32_t>(float_to_bf16_bits(v.y)) << 16);
-  o.y = static_cast<uint32_t>(float_to_bf16_bits(v.z)) | (static_cast<uint32_t>(float_to_bf16_bits(v.w)) << 16);
-  return o;
-}
-
-__device__ __forceinline__ float4 unpack_bf16x4(const uint2& u) {
-  return make_float4(bf16_bits_to_float(u.x & 0xffffu), bf16_bits_to_float(u.x >> 16),
-                     bf16_bits_to_float(u.y & 0xffffu), bf16_bits_to_float(u.y >> 16));
-}
-
-// scalar head / tail element of a shard range handled by thread t of CTA 0 (or ~0)
-__device__ __forceinline__ uint64_t edge_element(const ShardRange& r, unsigned t) {
-  const uint64_t nhead = r.head_end - r.lo, ntail = r.hi - r.tail_begin;
-  if (t < nhead) return r.lo + t;
-  if (t - nhead < ntail) return r.tail_begin + (t - nhead);
-  return ~0ull;
-}
-
 // N = compile-time world size (2..8), 0 = run-time world (<= kMaxRanks)
 template <int N, bool BF16>
 __global__ void __launch_bounds__(kPushThreads, 2) fused_sync_sgd_push_kernel(const SyncParams p) {
@@ -91,7 +69,6 @@ __global__ void __launch_bounds__(kPushThreads, 2) fused_sync_sgd_push_kernel(co
   const uint64_t slot = p.recv_stride;
   float* g = const_cast<float*>(p.diff[rank]);
   const bool zero = p.zero_diff != 0;
-  const float4 z4 = make_float4(0.f, 0.f, 0.f, 0.f);
 
   // ---- phase 1: scatter my gradient into the owners' receive slots ----------
   // Destinations are staggered (rank+1, rank+2, ...), so at any moment the ranks target different peers.  For a
@@ -109,9 +86,7 @@ __global__ void __launch_bounds__(kPushThreads, 2) fused_sync_sgd_push_kernel(co
         const uint64_t j = j0 + static_cast<uint64_t>(u) * stride;
 #pragma unroll
         for (int d = 0; d < D; ++d) {
-          int q = rank + 1 + d;
-          if (q >= N) q -= N;
-          const ShardRange r = shard_range(p.count, N, q);
+          const ShardRange r = shard_range(p.count, N, peer(rank, 1 + d, N));
           const uint64_t i = vec_elem(r, j);
           if (i != ~0ull) v[u][d] = ld_stream(g + i);
         }
@@ -121,8 +96,7 @@ __global__ void __launch_bounds__(kPushThreads, 2) fused_sync_sgd_push_kernel(co
         const uint64_t j = j0 + static_cast<uint64_t>(u) * stride;
 #pragma unroll
         for (int d = 0; d < D; ++d) {
-          int q = rank + 1 + d;
-          if (q >= N) q -= N;
+          const int q = peer(rank, 1 + d, N);
           const ShardRange r = shard_range(p.count, N, q);
           const uint64_t i = vec_elem(r, j), base = r.vec_base << 2;  // slot element 0 <-> global element base
           if (i != ~0ull) {
@@ -139,8 +113,7 @@ __global__ void __launch_bounds__(kPushThreads, 2) fused_sync_sgd_push_kernel(co
     }
   } else {
     for (int d = 1; d < world; ++d) {
-      int q = rank + d;
-      if (q >= world) q -= world;
+      const int q = peer(rank, d, world);
       const ShardRange r = shard_range(p.count, world, q);
       const uint64_t base = r.vec_base << 2;
       for (uint64_t j = tid; j < r.off + r.nvec; j += stride) {
@@ -159,8 +132,7 @@ __global__ void __launch_bounds__(kPushThreads, 2) fused_sync_sgd_push_kernel(co
   }
   if (blockIdx.x == 0) {  // scalar head / tail elements of every foreign shard
     for (int d = 1; d < world; ++d) {
-      int q = rank + d;
-      if (q >= world) q -= world;
+      const int q = peer(rank, d, world);
       const ShardRange r = shard_range(p.count, world, q);
       const uint64_t base = r.vec_base << 2;
       const uint64_t i = edge_element(r, threadIdx.x);
@@ -175,19 +147,7 @@ __global__ void __launch_bounds__(kPushThreads, 2) fused_sync_sgd_push_kernel(co
   // ---- barrier A: every contribution to my shard has landed -----------------
   cta_signal(p, 0);
   if (zero) {  // ClearParamDiffs of what this CTA pushed, hidden in the flag flight
-    for (int d = 1; d < world; ++d) {
-      int q = rank + d;
-      if (q >= world) q -= world;
-      const ShardRange r = shard_range(p.count, world, q);
-      for (uint64_t j = tid; j < r.off + r.nvec; j += stride) {
-        const uint64_t i = vec_elem(r, j);
-        if (i != ~0ull) st_vec(g + i, z4);
-      }
-      if (blockIdx.x == 0) {
-        const uint64_t i = edge_element(r, threadIdx.x);
-        if (i != ~0ull) g[i] = 0.f;
-      }
-    }
+    for (int d = 1; d < world; ++d) zero_range<true>(g, shard_range(p.count, world, peer(rank, d, world)), tid, stride);
   }
   if (!cta_wait(p, 0, &s_abort)) return;
   if (tracer) p.trace[2] = globaltimer_ns();
@@ -279,28 +239,14 @@ __global__ void __launch_bounds__(kPushThreads, 2) fused_sync_sgd_push_kernel(co
     if (blockIdx.x == 0) {  // scalar head / tail of my shard
       const uint64_t i = edge_element(r, threadIdx.x);
       if (i != ~0ull) {
-        SegCursor c2 = cur;
-        c2.seek(i);
-        float x = g[i];
-        if (BF16) x = round_bf16(x);
-        float acc = __fmul_rn(inv, x);
+        float acc = scaled(inv, BF16 ? round_bf16(g[i]) : g[i]);
         for (int k = 1; k < world; ++k) {
-          int src = rank + k;
-          if (src >= world) src -= world;
+          const int src = peer(rank, k, world);
           const float y = BF16 ? bf16_bits_to_float(static_cast<const uint16_t*>(p.recv[rank])[src * slot + (i - base)])
                                : static_cast<const float*>(p.recv[rank])[src * slot + (i - base)];
-          acc = __fadd_rn(__fmul_rn(inv, y), acc);
+          add_scaled(acc, inv, y);
         }
-        float w = wl[i], h = hl[i];
-        sgd_element(acc, w, h, __fmul_rn(p.rate, c2.lr_mult[c2.k]), __fmul_rn(p.weight_decay, c2.decay_mult[c2.k]),
-                    p.momentum, p.l1);
-        hl[i] = h;
-        wl[i] = w;
-        for (int k = 1; k < world; ++k) {
-          int dst = rank + k;
-          if (dst >= world) dst -= world;
-          p.data[dst][i] = w;
-        }
+        store_peers(p, world, i, sgd_scalar(p, cur, i, acc, wl, hl));
       }
     }
   }
@@ -309,25 +255,10 @@ __global__ void __launch_bounds__(kPushThreads, 2) fused_sync_sgd_push_kernel(co
   // ---- barrier B: every peer's weight shard has landed in my data_ ----------
   cta_signal(p, 1);
   if (zero) {  // own shard of diff_: read by this CTA in phase 2 only
-    const ShardRange r = shard_range(p.count, world, rank);
-    for (uint64_t j = tid; j < r.off + r.nvec; j += stride) {
-      const uint64_t i = vec_elem(r, j);
-      if (i != ~0ull) st_vec(g + i, z4);
-    }
-    if (blockIdx.x == 0) {
-      const uint64_t i = edge_element(r, threadIdx.x);
-      if (i != ~0ull) g[i] = 0.f;
-    }
+    zero_range<true>(g, shard_range(p.count, world, rank), tid, stride);
   }
   if (!cta_wait(p, 1, &s_abort)) return;
   if (tracer) p.trace[4] = globaltimer_ns();
-}
-
-template <int N>
-cudaError_t launch_push_n(const SyncParams& p, int grid, int block, size_t smem, cudaStream_t stream) {
-  if (p.grad_bf16) fused_sync_sgd_push_kernel<N, true><<<grid, block, smem, stream>>>(p);
-  else fused_sync_sgd_push_kernel<N, false><<<grid, block, smem, stream>>>(p);
-  return cudaGetLastError();
 }
 
 }  // namespace
@@ -339,7 +270,7 @@ uint64_t push_recv_stride(uint64_t count, int world) {
 
 cudaError_t launch_fused_sync_sgd_push(const SyncParams& p, int grid, int block, int vecs_per_thread,
                                        cudaStream_t stream) {
-  if (p.world < 2 || p.world > kMaxRanks || p.rank < 0 || p.rank >= p.world) return cudaErrorInvalidValue;
+  if (!check_world(p, 2)) return cudaErrorInvalidValue;
   if (p.mode != kModeTwoShot || p.recv_stride == 0) return cudaErrorInvalidValue;
   if (block <= 0) block = kPushThreads;
   if (block > kPushThreads || block < kMaxRanks || (block & 31)) return cudaErrorInvalidValue;
@@ -356,17 +287,12 @@ cudaError_t launch_fused_sync_sgd_push(const SyncParams& p, int grid, int block,
     grid = static_cast<int>(need > static_cast<uint64_t>(cap) ? cap : need);
   }
   if (grid > kMaxCtas) grid = kMaxCtas;
-  const size_t smem = p.nseg <= kPushMaxSeg ? static_cast<size_t>(p.nseg) * (sizeof(uint64_t) + 2 * sizeof(float)) : 0;
-  switch (p.world) {
-    case 2: return launch_push_n<2>(p, grid, block, smem, stream);
-    case 3: return launch_push_n<3>(p, grid, block, smem, stream);
-    case 4: return launch_push_n<4>(p, grid, block, smem, stream);
-    case 5: return launch_push_n<5>(p, grid, block, smem, stream);
-    case 6: return launch_push_n<6>(p, grid, block, smem, stream);
-    case 7: return launch_push_n<7>(p, grid, block, smem, stream);
-    case 8: return launch_push_n<8>(p, grid, block, smem, stream);
-    default: return launch_push_n<0>(p, grid, block, smem, stream);
-  }
+  const size_t smem = seg_smem_bytes(p, kPushMaxSeg);
+  return dispatch_world(p.world, [&](auto N) {
+    if (p.grad_bf16) fused_sync_sgd_push_kernel<N, true><<<grid, block, smem, stream>>>(p);
+    else fused_sync_sgd_push_kernel<N, false><<<grid, block, smem, stream>>>(p);
+    return cudaGetLastError();
+  });
 }
 
 }  // namespace cosb

@@ -177,12 +177,7 @@ fused_sync_sgd_tma_kernel(const SyncParams p, const int tile_elems) {
 
   // smem carve-up: [full mbarriers][segment table][stages]
   uint64_t* full = reinterpret_cast<uint64_t*>(smem);
-  uint64_t* s_end = reinterpret_cast<uint64_t*>(smem + 128);
-  const bool seg_in_smem = p.nseg <= kMaxSegSmemTma;
-  const int nseg_s = seg_in_smem ? p.nseg : 0;
-  float* s_lr = reinterpret_cast<float*>(s_end + nseg_s);
-  float* s_dm = s_lr + nseg_s;
-  size_t off = 128 + static_cast<size_t>(nseg_s) * 16;
+  size_t off = 128 + (p.nseg <= kMaxSegSmemTma ? static_cast<size_t>(p.nseg) * 16 : 0);
   off = (off + 127) & ~static_cast<size_t>(127);
   const size_t src_bytes = static_cast<size_t>(nsrc) * tile_elems * gsz;
   const size_t stage_bytes = src_bytes + 2ull * tile_elems * sizeof(float);
@@ -199,18 +194,8 @@ fused_sync_sgd_tma_kernel(const SyncParams p, const int tile_elems) {
     for (int k = 0; k < kStages; ++k) mbar_init(&full[k], 1);
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
   }
-  for (int k = tid; k < nseg_s; k += kTmaThreads) {
-    s_end[k] = p.seg_end[k];
-    s_lr[k] = p.seg_lr_mult[k];
-    s_dm[k] = p.seg_decay_mult[k];
-  }
+  SegCursor cur = load_seg_table(p, smem + 128, kMaxSegSmemTma);
   __syncthreads();
-  SegCursor cur;
-  cur.end = seg_in_smem ? s_end : p.seg_end;
-  cur.lr_mult = seg_in_smem ? s_lr : p.seg_lr_mult;
-  cur.decay_mult = seg_in_smem ? s_dm : p.seg_decay_mult;
-  cur.nseg = p.nseg;
-  cur.k = 0;
   bool cur_seeked = false;
 
   // ---- phase 0: fp32 -> bf16 wire cast, same tile -> CTA partition ----------
@@ -224,17 +209,12 @@ fused_sync_sgd_tma_kernel(const SyncParams p, const int tile_elems) {
            t0 += static_cast<uint64_t>(gridDim.x) * tile_elems) {
         const uint64_t t1 = (t0 + tile_elems < body1) ? t0 + tile_elems : body1;
         for (uint64_t i = t0 + 4ull * tid; i < t1; i += 4ull * kTmaThreads) {
-          float4 v = ld_stream(g + i);
-          uint2 o;
-          o.x = static_cast<uint32_t>(float_to_bf16_bits(v.x)) | (static_cast<uint32_t>(float_to_bf16_bits(v.y)) << 16);
-          o.y = static_cast<uint32_t>(float_to_bf16_bits(v.z)) | (static_cast<uint32_t>(float_to_bf16_bits(v.w)) << 16);
-          *reinterpret_cast<uint2*>(wv + i) = o;
+          *reinterpret_cast<uint2*>(wv + i) = pack_bf16x4(ld_stream(g + i));
         }
       }
       if (blockIdx.x == 0) {
-        const uint64_t nhead = r.head_end - r.lo, ntail = r.hi - r.tail_begin;
-        if (tid < nhead) wv[r.lo + tid] = float_to_bf16_bits(g[r.lo + tid]);
-        else if (tid - nhead < ntail) wv[r.tail_begin + (tid - nhead)] = float_to_bf16_bits(g[r.tail_begin + (tid - nhead)]);
+        const uint64_t i = edge_element(r, tid);
+        if (i != ~0ull) wv[i] = float_to_bf16_bits(g[i]);
       }
     }
   }
@@ -255,8 +235,7 @@ fused_sync_sgd_tma_kernel(const SyncParams p, const int tile_elems) {
     const uint64_t i0 = j.elem0();
     mbar_expect_tx(&full[k], n * (static_cast<uint32_t>(nsrc) * gsz + 8u));
     for (int q = 0; q < nsrc; ++q) {
-      int src = j.s + q;
-      if (src >= world) src -= world;
+      const int src = peer(j.s, q, world);
       const void* g = local ? static_cast<const void*>(p.diff[rank] + i0)
                             : (BF16 ? static_cast<const void*>(p.wire[src] + i0)
                                     : static_cast<const void*>(p.diff[src] + i0));
@@ -298,32 +277,16 @@ fused_sync_sgd_tma_kernel(const SyncParams p, const int tile_elems) {
       float4 acc;
       if (local) {
         acc = *reinterpret_cast<const float4*>(v.src + static_cast<size_t>(e) * 4);
-        if (BF16) {
-          acc.x = bf16_bits_to_float(float_to_bf16_bits(acc.x));
-          acc.y = bf16_bits_to_float(float_to_bf16_bits(acc.y));
-          acc.z = bf16_bits_to_float(float_to_bf16_bits(acc.z));
-          acc.w = bf16_bits_to_float(float_to_bf16_bits(acc.w));
-        }
+        if (BF16) acc = round_bf16x4(acc);
       } else {
         const float inv = p.inv_scale;
         for (int q = 0; q < nsrc; ++q) {  // order s, s+1, ... (mod N): tile q holds rank (s+q)%N
           float4 x;
           const unsigned char* base = v.src + static_cast<size_t>(q) * tile_elems * gsz;
-          if (BF16) {
-            const uint2 u = *reinterpret_cast<const uint2*>(base + static_cast<size_t>(e) * 2);
-            x = make_float4(bf16_bits_to_float(u.x & 0xffffu), bf16_bits_to_float(u.x >> 16),
-                            bf16_bits_to_float(u.y & 0xffffu), bf16_bits_to_float(u.y >> 16));
-          } else {
-            x = *reinterpret_cast<const float4*>(base + static_cast<size_t>(e) * 4);
-          }
-          if (q == 0) {
-            acc = make_float4(__fmul_rn(inv, x.x), __fmul_rn(inv, x.y), __fmul_rn(inv, x.z), __fmul_rn(inv, x.w));
-          } else {
-            acc.x = __fadd_rn(__fmul_rn(inv, x.x), acc.x);
-            acc.y = __fadd_rn(__fmul_rn(inv, x.y), acc.y);
-            acc.z = __fadd_rn(__fmul_rn(inv, x.z), acc.z);
-            acc.w = __fadd_rn(__fmul_rn(inv, x.w), acc.w);
-          }
+          if (BF16) x = unpack_bf16x4(*reinterpret_cast<const uint2*>(base + static_cast<size_t>(e) * 2));
+          else x = *reinterpret_cast<const float4*>(base + static_cast<size_t>(e) * 4);
+          if (q == 0) acc = scaled(inv, x);
+          else add_scaled(acc, inv, x);
         }
       }
       float4 w = *reinterpret_cast<const float4*>(v.w + e);
@@ -343,11 +306,7 @@ fused_sync_sgd_tma_kernel(const SyncParams p, const int tile_elems) {
       tma_store(wl + i0, v.w, n * 4u);
       tma_store(hl + i0, v.h, n * 4u);
       if (push) {
-        for (int q = 1; q < world; ++q) {
-          int dst = rank + q;
-          if (dst >= world) dst -= world;
-          tma_store(p.data[dst] + i0, v.w, n * 4u);
-        }
+        for (int q = 1; q < world; ++q) tma_store(p.data[peer(rank, q, world)] + i0, v.w, n * 4u);
       }
       tma_commit();
       // the stage used by the PREVIOUS iteration is free once its stores have
@@ -370,39 +329,23 @@ fused_sync_sgd_tma_kernel(const SyncParams p, const int tile_elems) {
     const int s_last = (p.mode == kModeOneShot) ? world - 1 : (local ? 0 : rank);
     for (int s = s_first; s <= s_last; ++s) {
       const BodyRange r = body_range(p, s, A);
-      const uint64_t nhead = r.head_end - r.lo, ntail = r.hi - r.tail_begin;
-      uint64_t i = ~0ull;
-      if (tid < nhead) i = r.lo + tid;
-      else if (tid - nhead < ntail) i = r.tail_begin + (tid - nhead);
+      const uint64_t i = edge_element(r, tid);
       if (i != ~0ull) {
-        SegCursor c2 = cur;
-        c2.seek(i);
         float g;
         if (local) {
           g = p.diff[rank][i];
-          if (BF16) g = bf16_bits_to_float(float_to_bf16_bits(g));
+          if (BF16) g = round_bf16(g);
         } else {
           g = 0.f;
           for (int q = 0; q < world; ++q) {
-            int src = s + q;
-            if (src >= world) src -= world;
-            float x = BF16 ? bf16_bits_to_float(p.wire[src][i]) : p.diff[src][i];
-            x = __fmul_rn(p.inv_scale, x);
-            g = (q == 0) ? x : __fadd_rn(x, g);
+            const int src = peer(s, q, world);
+            const float x = BF16 ? bf16_bits_to_float(p.wire[src][i]) : p.diff[src][i];
+            if (q == 0) g = scaled(p.inv_scale, x);
+            else add_scaled(g, p.inv_scale, x);
           }
         }
-        float w = wl[i], h = hl[i];
-        sgd_element(g, w, h, __fmul_rn(p.rate, c2.lr_mult[c2.k]), __fmul_rn(p.weight_decay, c2.decay_mult[c2.k]),
-                    p.momentum, p.l1);
-        hl[i] = h;
-        wl[i] = w;
-        if (push) {
-          for (int q = 1; q < world; ++q) {
-            int dst = rank + q;
-            if (dst >= world) dst -= world;
-            p.data[dst][i] = w;
-          }
-        }
+        const float w = sgd_scalar(p, cur, i, g, wl, hl);
+        if (push) store_peers(p, world, i, w);
       }
     }
   }
@@ -425,11 +368,7 @@ fused_sync_sgd_tma_kernel(const SyncParams p, const int tile_elems) {
         const uint64_t t1 = (t0 + tile_elems < body1) ? t0 + tile_elems : body1;
         for (uint64_t i = t0 + 4ull * tid; i < t1; i += 4ull * kTmaThreads) *reinterpret_cast<float4*>(g + i) = z;
       }
-      if (blockIdx.x == 0) {
-        const uint64_t nhead = r.head_end - r.lo, ntail = r.hi - r.tail_begin;
-        if (tid < nhead) g[r.lo + tid] = 0.f;
-        else if (tid - nhead < ntail) g[r.tail_begin + (tid - nhead)] = 0.f;
-      }
+      zero_edges(g, r);
     }
   }
 }
@@ -437,13 +376,8 @@ fused_sync_sgd_tma_kernel(const SyncParams p, const int tile_elems) {
 }  // namespace
 
 cudaError_t launch_fused_sync_sgd_tma(const SyncParams& p, int grid, cudaStream_t stream) {
-  if (p.world < 1 || p.world > kMaxRanks || p.rank < 0 || p.rank >= p.world) return cudaErrorInvalidValue;
-  if (p.mode == kModeAllGather) return cudaErrorInvalidValue;
-  int dev = 0;
-  cudaGetDevice(&dev);
-  int sms = 148;
-  cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-  if (grid <= 0) grid = sms;  // persistent: one CTA per SM
+  if (!check_world(p, 1) || p.mode == kModeAllGather) return cudaErrorInvalidValue;
+  if (grid <= 0) grid = sm_count(-1);  // persistent: one CTA per SM
   if (grid > kMaxCtas) grid = kMaxCtas;
   const int nsrc = p.mode == kModeLocal ? 1 : p.world;
   const uint32_t gsz = (p.grad_bf16 && p.mode != kModeLocal) ? 2 : 4;
@@ -459,8 +393,7 @@ cudaError_t launch_fused_sync_sgd_tma(const SyncParams& p, int grid, cudaStream_
   if (p.zero_diff || p.grad_bf16) tiles = (p.count / (p.mode == kModeLocal ? 1 : p.world) + tile - 1) / tile;
   if (tiles < 1) tiles = 1;
   if (static_cast<uint64_t>(grid) > tiles) grid = static_cast<int>(tiles);
-  const int nseg_s = p.nseg <= kMaxSegSmemTma ? p.nseg : 0;
-  size_t smem = 128 + static_cast<size_t>(nseg_s) * 16;
+  size_t smem = 128 + seg_smem_bytes(p, kMaxSegSmemTma);
   smem = (smem + 127) & ~static_cast<size_t>(127);
   smem += static_cast<size_t>(kStages) * (per_elem * tile);
   smem += 128;

@@ -1,13 +1,21 @@
-// sync_device.cuh -- device-side building blocks shared by the two variants of
-// the fused sync kernel (fused_sync_sgd.cu: vector LDG/STG path,
-// fused_sync_sgd_tma.cu: cp.async.bulk pipeline): PTX wrappers, the per-CTA
-// cross-GPU barrier, the shard/vector partition, the blob (segment) cursor and
-// the SGD element update in the reference's operation order.
+// sync_device.cuh -- building blocks shared by the five variants of the fused
+// sync kernel (fused_sync_sgd.cu: LDG/STG pull, _tma.cu: cp.async.bulk pull,
+// _push.cu: stores only, _ll.cu: flag-in-data words, _nvls.cu: multimem):
+// PTX wrappers, bf16 pack / unpack / round, the ring order of the peers and the
+// scale-then-sum step of the reduction, the per-CTA cross-GPU barrier, the
+// shard/vector partition and its scalar head / tail, zeroing of diff_, the blob
+// (segment) cursor and its shared-memory copy, the SGD update of a vector and of
+// a scalar element in the reference's operation order, and the host side of
+// the launchers (argument check, SM count, world-size dispatch).  Not every
+// kernel uses every helper: where a helper changed a kernel's register
+// allocation, the kernel keeps its inline form (see DESIGN.md §3).
 #ifndef COS_SYNC_DEVICE_CUH_
 #define COS_SYNC_DEVICE_CUH_
 
 #include <cuda_bf16.h>
 #include <stdint.h>
+
+#include <type_traits>
 
 #include "fused_sync_sgd.hpp"
 
@@ -64,6 +72,64 @@ __device__ __forceinline__ float bf16_bits_to_float(uint32_t bits16) { return __
 
 __device__ __forceinline__ uint16_t float_to_bf16_bits(float f) {
   return __bfloat16_as_ushort(__float2bfloat16_rn(f));
+}
+
+// the value a gradient element has after crossing the bf16 wire
+__device__ __forceinline__ float round_bf16(float x) { return bf16_bits_to_float(float_to_bf16_bits(x)); }
+
+__device__ __forceinline__ float4 round_bf16x4(const float4& v) {
+  return make_float4(round_bf16(v.x), round_bf16(v.y), round_bf16(v.z), round_bf16(v.w));
+}
+
+__device__ __forceinline__ uint2 pack_bf16x4(const float4& v) {
+  uint2 o;
+  o.x = static_cast<uint32_t>(float_to_bf16_bits(v.x)) | (static_cast<uint32_t>(float_to_bf16_bits(v.y)) << 16);
+  o.y = static_cast<uint32_t>(float_to_bf16_bits(v.z)) | (static_cast<uint32_t>(float_to_bf16_bits(v.w)) << 16);
+  return o;
+}
+
+__device__ __forceinline__ float4 unpack_bf16x4(const uint2& u) {
+  return make_float4(bf16_bits_to_float(u.x & 0xffffu), bf16_bits_to_float(u.x >> 16),
+                     bf16_bits_to_float(u.y & 0xffffu), bf16_bits_to_float(u.y >> 16));
+}
+
+// ------------------------------------------------------- reduction order
+
+// The rank k places after `rank` on the ring (0 <= k < world).  Owner s sums the sources s, s+1, ... (mod N)
+// in that order (socket_sync_cpu.cpp:108-133); pushes go to rank+1, rank+2, ... so that at any moment the
+// ranks target different peers.
+__device__ __forceinline__ int peer(int rank, int k, int world) {
+  int x = rank + k;
+  if (x >= world) x -= world;
+  return x;
+}
+
+// Every gradient is scaled by 1/N BEFORE the sum (parallel_cpu.cpp:120-122 runs before
+// socket_sync_cpu.cpp:112-132): acc = inv*x for the first source, acc = inv*x + acc for each later one.
+__device__ __forceinline__ float scaled(float inv, float x) { return __fmul_rn(inv, x); }
+
+__device__ __forceinline__ float4 scaled(float inv, const float4& x) {
+  return make_float4(__fmul_rn(inv, x.x), __fmul_rn(inv, x.y), __fmul_rn(inv, x.z), __fmul_rn(inv, x.w));
+}
+
+__device__ __forceinline__ void add_scaled(float& acc, float inv, float x) { acc = __fadd_rn(__fmul_rn(inv, x), acc); }
+
+__device__ __forceinline__ void add_scaled(float4& acc, float inv, const float4& x) {
+  acc.x = __fadd_rn(__fmul_rn(inv, x.x), acc.x);
+  acc.y = __fadd_rn(__fmul_rn(inv, x.y), acc.y);
+  acc.z = __fadd_rn(__fmul_rn(inv, x.z), acc.z);
+  acc.w = __fadd_rn(__fmul_rn(inv, x.w), acc.w);
+}
+
+// f(k) for k = 1 .. world-1, unrolled when the world size N is known at compile time (N = 0: run time)
+template <int N, class F>
+__device__ __forceinline__ void for_peers(int world, F&& f) {
+  if (N > 0) {
+#pragma unroll
+    for (int k = 1; k < (N > 0 ? N : 1); ++k) f(k);
+  } else {
+    for (int k = 1; k < world; ++k) f(k);
+  }
 }
 
 // ------------------------------------------------------ cross-GPU barrier
@@ -183,6 +249,42 @@ __device__ __forceinline__ ShardRange shard_range(uint64_t count, int world, int
   return r;
 }
 
+// Scalar head / tail element of range r handled by thread t of CTA 0, or ~0.  R is ShardRange or any range with
+// the same lo / head_end / tail_begin / hi fields.
+template <class R>
+__device__ __forceinline__ uint64_t edge_element(const R& r, unsigned t) {
+  const uint64_t nhead = r.head_end - r.lo, ntail = r.hi - r.tail_begin;
+  if (t < nhead) return r.lo + t;
+  if (t - nhead < ntail) return r.tail_begin + (t - nhead);
+  return ~0ull;
+}
+
+// diff_ := 0 over the scalar head / tail of range r (CTA 0)
+template <class R>
+__device__ __forceinline__ void zero_edges(float* g, const R& r) {
+  if (blockIdx.x == 0) {
+    const uint64_t i = edge_element(r, threadIdx.x);
+    if (i != ~0ull) g[i] = 0.f;
+  }
+}
+
+// diff_ := 0 over shard range r with st_vec, which stays ordered behind the asm loads of the same words before it:
+// the float4 body in the plain j = tid + k*stride walk (kAligned = false) or the 512-byte aligned vec_elem walk,
+// then the scalar head / tail.
+template <bool kAligned>
+__device__ __forceinline__ void zero_range(float* g, const ShardRange& r, uint64_t tid, uint64_t stride) {
+  const float4 z = make_float4(0.f, 0.f, 0.f, 0.f);
+  if (kAligned) {
+    for (uint64_t j = tid; j < r.off + r.nvec; j += stride) {
+      const uint64_t i = vec_elem(r, j);
+      if (i != ~0ull) st_vec(g + i, z);
+    }
+  } else {
+    for (uint64_t j = tid; j < r.nvec; j += stride) st_vec(g + ((r.vec_lo + j) << 2), z);
+  }
+  zero_edges(g, r);
+}
+
 // ----------------------------------------------------------- SGD element
 
 struct SegCursor {
@@ -203,6 +305,29 @@ struct SegCursor {
     while (k < nseg - 1 && i >= end[k]) ++k;
   }
 };
+
+// Copies the segment table to shared memory at smem when it has at most max_seg entries (otherwise the cursor
+// reads global memory) and returns a cursor over it.  The CTA must __syncthreads() before the first seek.
+__device__ __forceinline__ SegCursor load_seg_table(const SyncParams& p, unsigned char* smem, int max_seg) {
+  uint64_t* s_end = reinterpret_cast<uint64_t*>(smem);
+  float* s_lr = reinterpret_cast<float*>(s_end + p.nseg);
+  float* s_dm = s_lr + p.nseg;
+  const bool in_smem = p.nseg <= max_seg;
+  if (in_smem) {
+    for (int k = threadIdx.x; k < p.nseg; k += blockDim.x) {
+      s_end[k] = p.seg_end[k];
+      s_lr[k] = p.seg_lr_mult[k];
+      s_dm[k] = p.seg_decay_mult[k];
+    }
+  }
+  SegCursor c;
+  c.end = in_smem ? s_end : p.seg_end;
+  c.lr_mult = in_smem ? s_lr : p.seg_lr_mult;
+  c.decay_mult = in_smem ? s_dm : p.seg_decay_mult;
+  c.nseg = p.nseg;
+  c.k = 0;
+  return c;
+}
 
 // Regularize + ComputeUpdateValue + Blob::Update for one element, in the
 // reference's operation order with one rounding per operation:
@@ -262,6 +387,62 @@ __device__ __forceinline__ void sgd_vec(const SyncParams& p, SegCursor& c, uint6
   }
 }
 
+// Scalar (head / tail) element i with reduced gradient g: update with its blob's multipliers (c is sought from
+// scratch), store h and w locally, return the new weight.
+__device__ __forceinline__ float sgd_scalar(const SyncParams& p, SegCursor c, uint64_t i, float g, float* wl,
+                                            float* hl) {
+  c.seek(i);
+  float w = wl[i], h = hl[i];
+  sgd_element(g, w, h, __fmul_rn(p.rate, c.lr_mult[c.k]), __fmul_rn(p.weight_decay, c.decay_mult[c.k]), p.momentum,
+              p.l1);
+  hl[i] = h;
+  wl[i] = w;
+  return w;
+}
+
+// the all-gather of one scalar weight: element i of every peer's data_
+__device__ __forceinline__ void store_peers(const SyncParams& p, int world, uint64_t i, float w) {
+  for (int k = 1; k < world; ++k) p.data[peer(p.rank, k, world)][i] = w;
+}
+
+// -------------------------------------------------------------- host side
+
+// world / rank of a launch; kernels that exchange data with peers ask for min_world = 2
+inline bool check_world(const SyncParams& p, int min_world) {
+  return p.world >= min_world && p.world <= kMaxRanks && p.rank >= 0 && p.rank < p.world;
+}
+
+// SMs of `device` (-1: the current device); 148 (B200) if the query fails
+inline int sm_count(int device) {
+  int sms = 0;
+  if ((device < 0 && cudaGetDevice(&device) != cudaSuccess) ||
+      cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device) != cudaSuccess || sms <= 0) {
+    cudaGetLastError();
+    sms = 148;
+  }
+  return sms;
+}
+
+// dynamic shared memory of a segment table the kernel copies into shared memory when nseg <= max_seg
+inline size_t seg_smem_bytes(const SyncParams& p, int max_seg) {
+  return p.nseg <= max_seg ? static_cast<size_t>(p.nseg) * (sizeof(uint64_t) + 2 * sizeof(float)) : 0;
+}
+
+// f(std::integral_constant<int, N>()) with N = world for the world sizes 2..8 the kernels are compiled for,
+// N = 0 (world size known at run time only) for every other value
+template <class F>
+cudaError_t dispatch_world(int world, F&& f) {
+  switch (world) {
+    case 2: return f(std::integral_constant<int, 2>());
+    case 3: return f(std::integral_constant<int, 3>());
+    case 4: return f(std::integral_constant<int, 4>());
+    case 5: return f(std::integral_constant<int, 5>());
+    case 6: return f(std::integral_constant<int, 6>());
+    case 7: return f(std::integral_constant<int, 7>());
+    case 8: return f(std::integral_constant<int, 8>());
+    default: return f(std::integral_constant<int, 0>());
+  }
+}
 
 }  // namespace
 }  // namespace cosb
