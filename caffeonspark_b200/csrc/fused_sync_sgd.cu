@@ -49,39 +49,12 @@ __device__ __forceinline__ float4 reduce_vec(const SyncParams& p, int s, uint64_
   float4 x[N];
 #pragma unroll
   for (int j = 0; j < N; ++j) {  // all loads first: N independent 128-bit requests in flight
-    int src = s + j;
-    if (src >= N) src -= N;
-    if (BF16) {
-      uint2 u = ld_stream_u2(p.wire[src] + i);
-      x[j] = make_float4(bf16_bits_to_float(u.x & 0xffffu), bf16_bits_to_float(u.x >> 16),
-                         bf16_bits_to_float(u.y & 0xffffu), bf16_bits_to_float(u.y >> 16));
-    } else {
-      x[j] = ld_stream(p.diff[src] + i);
-    }
+    const int src = peer(s, j, N);
+    x[j] = BF16 ? unpack_bf16x4(ld_stream_u2(p.wire[src] + i)) : ld_stream(p.diff[src] + i);
   }
-  const float inv = p.inv_scale;
-  float4 acc = make_float4(__fmul_rn(inv, x[0].x), __fmul_rn(inv, x[0].y), __fmul_rn(inv, x[0].z),
-                           __fmul_rn(inv, x[0].w));
+  float4 acc = scaled(p.inv_scale, x[0]);
 #pragma unroll
-  for (int j = 1; j < N; ++j) {
-    acc.x = __fadd_rn(__fmul_rn(inv, x[j].x), acc.x);
-    acc.y = __fadd_rn(__fmul_rn(inv, x[j].y), acc.y);
-    acc.z = __fadd_rn(__fmul_rn(inv, x[j].z), acc.z);
-    acc.w = __fadd_rn(__fmul_rn(inv, x[j].w), acc.w);
-  }
-  return acc;
-}
-
-// runtime-world fallback (N not instantiated): sequential accumulate
-template <bool BF16>
-__device__ __forceinline__ float reduce_scalar(const SyncParams& p, int s, uint64_t i) {
-  float acc = 0.f;
-  for (int j = 0; j < p.world; ++j) {
-    const int src = peer(s, j, p.world);
-    const float x = BF16 ? bf16_bits_to_float(p.wire[src][i]) : p.diff[src][i];
-    if (j == 0) acc = scaled(p.inv_scale, x);
-    else add_scaled(acc, p.inv_scale, x);
-  }
+  for (int j = 1; j < N; ++j) add_scaled(acc, p.inv_scale, x[j]);
   return acc;
 }
 
@@ -100,26 +73,9 @@ template <int N, bool BF16>
 __global__ void __launch_bounds__(kDefaultThreads, 2) fused_sync_sgd_kernel(const SyncParams p) {
   extern __shared__ unsigned char smem_raw[];
   __shared__ int s_abort;
-  // segment (= learnable blob) table into shared memory
-  uint64_t* s_end = reinterpret_cast<uint64_t*>(smem_raw);
-  float* s_lr = reinterpret_cast<float*>(s_end + p.nseg);
-  float* s_dm = s_lr + p.nseg;
-  const bool seg_in_smem = p.nseg <= kMaxSegSmem;
-  if (seg_in_smem) {
-    for (int k = threadIdx.x; k < p.nseg; k += blockDim.x) {
-      s_end[k] = p.seg_end[k];
-      s_lr[k] = p.seg_lr_mult[k];
-      s_dm[k] = p.seg_decay_mult[k];
-    }
-  }
+  SegCursor cur = load_seg_table(p, smem_raw, kMaxSegSmem);  // segment (= learnable blob) table
   if (threadIdx.x == 0) s_abort = 0;
   __syncthreads();
-  SegCursor cur;
-  cur.end = seg_in_smem ? s_end : p.seg_end;
-  cur.lr_mult = seg_in_smem ? s_lr : p.seg_lr_mult;
-  cur.decay_mult = seg_in_smem ? s_dm : p.seg_decay_mult;
-  cur.nseg = p.nseg;
-  cur.k = 0;
 
   const bool tracer = p.trace != nullptr && blockIdx.x == 0 && threadIdx.x == 0;
   if (tracer) p.trace[0] = globaltimer_ns();
@@ -160,25 +116,11 @@ __global__ void __launch_bounds__(kDefaultThreads, 2) fused_sync_sgd_kernel(cons
     for (uint64_t j = tid; j < r.nvec; j += stride) {
       const uint64_t i = (r.vec_lo + j) << 2;
       const float4 v = ld_stream(w + i);
-      for (int q = 1; q < world; ++q) {
-        int dst = rank + q;
-        if (dst >= world) dst -= world;
-        st_vec(p.data[dst] + i, v);
-      }
+      for (int q = 1; q < world; ++q) st_vec(p.data[peer(rank, q, world)] + i, v);
     }
     if (blockIdx.x == 0) {
-      const uint64_t nhead = r.head_end - r.lo, ntail = r.hi - r.tail_begin;
-      uint64_t i = ~0ull;
-      if (threadIdx.x < nhead) i = r.lo + threadIdx.x;
-      else if (threadIdx.x - nhead < ntail) i = r.tail_begin + (threadIdx.x - nhead);
-      if (i != ~0ull) {
-        const float v = w[i];
-        for (int q = 1; q < world; ++q) {
-          int dst = rank + q;
-          if (dst >= world) dst -= world;
-          p.data[dst][i] = v;
-        }
-      }
+      const uint64_t i = edge_element(r, threadIdx.x);
+      if (i != ~0ull) store_peers(p, world, i, w[i]);
     }
   } else {
     // shards this rank updates: its own (two-shot), all (one-shot), [0,P) (local)
@@ -188,13 +130,7 @@ __global__ void __launch_bounds__(kDefaultThreads, 2) fused_sync_sgd_kernel(cons
     float* wl = p.data[rank];
     float* hl = p.hist;
     for (int s = s_first; s <= s_last; ++s) {
-      ShardRange r;
-      if (p.mode == kModeLocal) {
-        r.lo = 0; r.hi = p.count; r.vec_lo = 0; r.nvec = p.count >> 2;
-        r.head_end = 0; r.tail_begin = r.nvec << 2;
-      } else {
-        r = shard_range(p.count, world, s);
-      }
+      const ShardRange r = p.mode == kModeLocal ? shard_range(p.count, 1, 0) : shard_range(p.count, world, s);
       if (tid < r.nvec) cur.seek((r.vec_lo + tid) << 2);
       for (uint64_t j = tid; j < r.nvec; j += stride) {
         const uint64_t i = (r.vec_lo + j) << 2;
@@ -233,6 +169,7 @@ __global__ void __launch_bounds__(kDefaultThreads, 2) fused_sync_sgd_kernel(cons
 
   // ---- phase 2: ClearParamDiffs of the next Step --------------------------
   if (p.zero_diff && p.mode != kModeAllGather) {
+    // inline, not zero_range<false>: its asm stores are not unrolled (<5,false>: STG.E.128 36 -> 27 static)
     float* g = const_cast<float*>(p.diff[rank]);
     const float4 z = make_float4(0.f, 0.f, 0.f, 0.f);
     if (p.mode == kModeLocal) {

@@ -130,17 +130,7 @@ template <int N, bool BF16>
 __global__ void __launch_bounds__(kLLThreads, 1) fused_sync_sgd_ll_kernel(const SyncParams p) {
   extern __shared__ unsigned char smem_raw[];
   __shared__ int s_abort;
-  uint64_t* s_end = reinterpret_cast<uint64_t*>(smem_raw);
-  float* s_lr = reinterpret_cast<float*>(s_end + p.nseg);
-  float* s_dm = s_lr + p.nseg;
-  const bool seg_in_smem = p.nseg <= kLLMaxSeg;
-  if (seg_in_smem) {
-    for (int k = threadIdx.x; k < p.nseg; k += blockDim.x) {
-      s_end[k] = p.seg_end[k];
-      s_lr[k] = p.seg_lr_mult[k];
-      s_dm[k] = p.seg_decay_mult[k];
-    }
-  }
+  copy_seg_table(p, smem_raw, kLLMaxSeg);
   if (threadIdx.x == 0) s_abort = 0;
   __syncthreads();
   const bool tracer = p.trace != nullptr && blockIdx.x == 0 && threadIdx.x == 0;
@@ -168,23 +158,20 @@ __global__ void __launch_bounds__(kLLThreads, 1) fused_sync_sgd_ll_kernel(const 
     float4 v[D];
 #pragma unroll
     for (int d = 0; d < D; ++d) {
-      int q = rank + 1 + d;
-      if (q >= N) q -= N;
+      const int q = peer(rank, 1 + d, N);
       const ShardRange r = shard_range(p.count, N, q);
       if (j < r.nvec) v[d] = ld_stream(g + ((r.vec_lo + j) << 2));
     }
 #pragma unroll
     for (int d = 0; d < D; ++d) {
-      int q = rank + 1 + d;
-      if (q >= N) q -= N;
+      const int q = peer(rank, 1 + d, N);
       const ShardRange r = shard_range(p.count, N, q);
       if (j < r.nvec) {
         const uint64_t i = (r.vec_lo + j) << 2, base = r.lo & ~3ull;
         uint64_t* dst = p.ll_grad[q] + static_cast<uint64_t>(rank) * gslot;
         if (BF16) {
-          const uint32_t lo2 = static_cast<uint32_t>(float_to_bf16_bits(v[d].x)) | (static_cast<uint32_t>(float_to_bf16_bits(v[d].y)) << 16);
-          const uint32_t hi2 = static_cast<uint32_t>(float_to_bf16_bits(v[d].z)) | (static_cast<uint32_t>(float_to_bf16_bits(v[d].w)) << 16);
-          st_ll2(dst + ((i - base) >> 1), ll_word(lo2, flag), ll_word(hi2, flag));
+          const uint2 o = pack_bf16x4(v[d]);
+          st_ll2(dst + ((i - base) >> 1), ll_word(o.x, flag), ll_word(o.y, flag));
         } else {
           uint64_t* w = dst + (i - base);
           st_ll2(w, ll_word(__float_as_uint(v[d].x), flag), ll_word(__float_as_uint(v[d].y), flag));
@@ -195,13 +182,11 @@ __global__ void __launch_bounds__(kLLThreads, 1) fused_sync_sgd_ll_kernel(const 
   }
   if (blockIdx.x == 0) {
     for (int d = 1; d < world; ++d) {
-      int q = rank + d;
-      if (q >= world) q -= world;
+      const int q = peer(rank, d, world);
       const ShardRange r = shard_range(p.count, world, q);
       const uint64_t e = edge_element(r, threadIdx.x);
       if (e != ~0ull) {
-        float x = g[e];
-        if (BF16) x = bf16_bits_to_float(float_to_bf16_bits(x));
+        const float x = BF16 ? round_bf16(g[e]) : g[e];
         st_ll1(p.ll_grad[q] + static_cast<uint64_t>(rank) * gslot + gedge + edge_index(r, e), ll_word(__float_as_uint(x), flag));
       }
     }
@@ -213,12 +198,7 @@ __global__ void __launch_bounds__(kLLThreads, 1) fused_sync_sgd_ll_kernel(const 
   if (tracer) p.trace[2] = globaltimer_ns();
 
   // ---- phase 2: poll + reduce + update + push the new weights ----------------
-  SegCursor cur;
-  cur.end = seg_in_smem ? s_end : p.seg_end;
-  cur.lr_mult = seg_in_smem ? s_lr : p.seg_lr_mult;
-  cur.decay_mult = seg_in_smem ? s_dm : p.seg_decay_mult;
-  cur.nseg = p.nseg;
-  cur.k = 0;
+  SegCursor cur = seg_cursor(p, smem_raw, kLLMaxSeg);
   Poll poll(p, &s_abort);
   bool alive = true;
   {
@@ -234,19 +214,15 @@ __global__ void __launch_bounds__(kLLThreads, 1) fused_sync_sgd_ll_kernel(const 
       float4 x = ld_stream(g + i);
       float4 w = *reinterpret_cast<const float4*>(wl + i);
       float4 h = *reinterpret_cast<const float4*>(hl + i);
-      if (BF16) {
-        x.x = bf16_bits_to_float(float_to_bf16_bits(x.x)); x.y = bf16_bits_to_float(float_to_bf16_bits(x.y));
-        x.z = bf16_bits_to_float(float_to_bf16_bits(x.z)); x.w = bf16_bits_to_float(float_to_bf16_bits(x.w));
-      }
-      float4 acc = make_float4(__fmul_rn(inv, x.x), __fmul_rn(inv, x.y), __fmul_rn(inv, x.z), __fmul_rn(inv, x.w));
+      if (BF16) x = round_bf16x4(x);
+      float4 acc = scaled(inv, x);
       constexpr int K = N - 1;  // the N-1 slots, polled together
       constexpr int W = BF16 ? 2 : 4;
       const uint64_t* ptr[K];
       uint64_t words[K][W];
 #pragma unroll
       for (int k = 0; k < K; ++k) {
-        int src = rank + 1 + k;
-        if (src >= world) src -= world;
+        const int src = peer(rank, 1 + k, world);
         ptr[k] = mine + src * gslot + (BF16 ? ((i - base) >> 1) : (i - base));
       }
       alive = poll_groups<K, W>(ptr, (1u << K) - 1u, flag, poll, rank, words);
@@ -255,19 +231,14 @@ __global__ void __launch_bounds__(kLLThreads, 1) fused_sync_sgd_ll_kernel(const 
       for (int k = 0; k < K; ++k) {  // reference order: rank+1, rank+2, ... (mod N)
         float4 y;
         if (BF16) {
-          const uint32_t u0 = static_cast<uint32_t>(words[k][0]), u1 = static_cast<uint32_t>(words[k][1]);
-          y = make_float4(bf16_bits_to_float(u0 & 0xffffu), bf16_bits_to_float(u0 >> 16),
-                          bf16_bits_to_float(u1 & 0xffffu), bf16_bits_to_float(u1 >> 16));
+          y = unpack_bf16x4(make_uint2(static_cast<uint32_t>(words[k][0]), static_cast<uint32_t>(words[k][1])));
         } else {
           y = make_float4(__uint_as_float(static_cast<uint32_t>(words[k][0])),
                           __uint_as_float(static_cast<uint32_t>(words[k][1])),
                           __uint_as_float(static_cast<uint32_t>(words[k][W - 2])),
                           __uint_as_float(static_cast<uint32_t>(words[k][W - 1])));
         }
-        acc.x = __fadd_rn(__fmul_rn(inv, y.x), acc.x);
-        acc.y = __fadd_rn(__fmul_rn(inv, y.y), acc.y);
-        acc.z = __fadd_rn(__fmul_rn(inv, y.z), acc.z);
-        acc.w = __fadd_rn(__fmul_rn(inv, y.w), acc.w);
+        add_scaled(acc, inv, y);
       }
       if (!alive) break;
       sgd_vec(p, cur, i, acc, w, h);
@@ -276,8 +247,7 @@ __global__ void __launch_bounds__(kLLThreads, 1) fused_sync_sgd_ll_kernel(const 
       const uint64_t wa = ll_word(__float_as_uint(w.x), flag), wb = ll_word(__float_as_uint(w.y), flag);
       const uint64_t wc = ll_word(__float_as_uint(w.z), flag), wd = ll_word(__float_as_uint(w.w), flag);
       for (int k = 1; k < world; ++k) {
-        int dst = rank + k;
-        if (dst >= world) dst -= world;
+        const int dst = peer(rank, k, world);
         uint64_t* o = p.ll_weight[dst] + static_cast<uint64_t>(rank) * wslot + (i - base);
         st_ll2(o, wa, wb);
         st_ll2(o + 2, wc, wd);
@@ -286,27 +256,17 @@ __global__ void __launch_bounds__(kLLThreads, 1) fused_sync_sgd_ll_kernel(const 
     if (alive && blockIdx.x == 0) {  // scalar head / tail of my shard
       const uint64_t e = edge_element(r, threadIdx.x);
       if (e != ~0ull) {
-        SegCursor c2 = cur;
-        c2.seek(e);
-        float x = g[e];
-        if (BF16) x = bf16_bits_to_float(float_to_bf16_bits(x));
-        float acc = __fmul_rn(inv, x);
+        float acc = scaled(inv, BF16 ? round_bf16(g[e]) : g[e]);
         for (int k = 1; alive && k < world; ++k) {
-          int src = rank + k;
-          if (src >= world) src -= world;
+          const int src = peer(rank, k, world);
           uint32_t u;
           alive = poll1(mine + src * gslot + gedge + edge_index(r, e), flag, poll, src, u);
-          if (alive) acc = __fadd_rn(__fmul_rn(inv, __uint_as_float(u)), acc);
+          if (alive) add_scaled(acc, inv, __uint_as_float(u));
         }
         if (alive) {
-          float w = wl[e], h = hl[e];
-          sgd_element(acc, w, h, __fmul_rn(p.rate, c2.lr_mult[c2.k]), __fmul_rn(p.weight_decay, c2.decay_mult[c2.k]),
-                      p.momentum, p.l1);
-          hl[e] = h;
-          wl[e] = w;
+          const float w = sgd_scalar(p, cur, e, acc, wl, hl);
           for (int k = 1; k < world; ++k) {
-            int dst = rank + k;
-            if (dst >= world) dst -= world;
+            const int dst = peer(rank, k, world);
             st_ll1(p.ll_weight[dst] + static_cast<uint64_t>(rank) * wslot + wedge + edge_index(r, e),
                    ll_word(__float_as_uint(w), flag));
           }
@@ -330,8 +290,7 @@ __global__ void __launch_bounds__(kLLThreads, 1) fused_sync_sgd_ll_kernel(const 
       uint32_t live = 0;
 #pragma unroll
       for (int d = 0; d < D; ++d) {
-        int q = rank + 1 + d;
-        if (q >= N) q -= N;
+        const int q = peer(rank, 1 + d, N);
         const ShardRange r = shard_range(p.count, N, q);
         const bool in = j < r.nvec;
         idx[d] = (r.vec_lo + j) << 2;
@@ -351,8 +310,7 @@ __global__ void __launch_bounds__(kLLThreads, 1) fused_sync_sgd_ll_kernel(const 
     }
     if (alive && blockIdx.x == 0) {
       for (int d = 1; alive && d < world; ++d) {
-        int q = rank + d;
-        if (q >= world) q -= world;
+        const int q = peer(rank, d, world);
         const ShardRange r = shard_range(p.count, world, q);
         const uint64_t e = edge_element(r, threadIdx.x);
         if (e != ~0ull) {

@@ -139,29 +139,15 @@ __global__ void __launch_bounds__(kNvlsThreads, 1) fused_sync_sgd_nvls_kernel(co
       }
     }
     if (blockIdx.x == 0) {  // scalar head / tail of my shard (<= 3 elements each): plain P2P, reference order
-      const uint64_t nhead = r.head_end - r.lo, ntail = r.hi - r.tail_begin;
-      uint64_t i = ~0ull;
-      if (threadIdx.x < nhead) i = r.lo + threadIdx.x;
-      else if (threadIdx.x - nhead < ntail) i = r.tail_begin + (threadIdx.x - nhead);
+      const uint64_t i = edge_element(r, threadIdx.x);
       if (i != ~0ull) {
-        cur.seek(i);
+        // inline, not reduce_scalar<false>: that changes the static FMUL count of <4,1,4> (515 -> 491)
         float acc = 0.f;
         for (int k = 0; k < world; ++k) {
-          int src = rank + k;
-          if (src >= world) src -= world;
-          const float y = __fmul_rn(inv, p.diff[src][i]);
+          const float y = __fmul_rn(inv, p.diff[peer(rank, k, world)][i]);
           acc = (k == 0) ? y : __fadd_rn(y, acc);
         }
-        float w = wl[i], h = hl[i];
-        sgd_element(acc, w, h, __fmul_rn(p.rate, cur.lr_mult[cur.k]), __fmul_rn(p.weight_decay, cur.decay_mult[cur.k]),
-                    p.momentum, p.l1);
-        hl[i] = h;
-        wl[i] = w;
-        for (int k = 1; k < world; ++k) {
-          int dst = rank + k;
-          if (dst >= world) dst -= world;
-          p.data[dst][i] = w;
-        }
+        store_peers(p, world, i, sgd_scalar(p, cur, i, acc, wl, hl));
       }
     }
   } else if (p.zero_diff) {

@@ -42,6 +42,17 @@ namespace {
 constexpr int kPushThreads = 512;
 constexpr int kPushMaxSeg = 1024;
 
+__device__ __forceinline__ void st_vec_u2(uint16_t* p, const uint2& v) {
+  asm volatile("st.global.v2.u32 [%0], {%1,%2};" ::"l"(p), "r"(v.x), "r"(v.y) : "memory");
+}
+
+// Receive slot `src` (the gradient rank src sends) in rank q's receive buffer.  Slot element 0 stands for global
+// element vec_base * 4 of q's shard.  T = float, or uint16_t (bf16 bits) on the bf16 wire.
+template <class T>
+__device__ __forceinline__ T* recv_slot(const SyncParams& p, int q, int src) {
+  return static_cast<T*>(p.recv[q]) + static_cast<uint64_t>(src) * p.recv_stride;
+}
+
 // N = compile-time world size (2..8), 0 = run-time world (<= kMaxRanks)
 template <int N, bool BF16>
 __global__ void __launch_bounds__(kPushThreads, 2) fused_sync_sgd_push_kernel(const SyncParams p) {
@@ -66,7 +77,6 @@ __global__ void __launch_bounds__(kPushThreads, 2) fused_sync_sgd_push_kernel(co
   const int rank = p.rank;
   const uint64_t tid = static_cast<uint64_t>(blockIdx.x) * blockDim.x + threadIdx.x;
   const uint64_t stride = static_cast<uint64_t>(gridDim.x) * blockDim.x;
-  const uint64_t slot = p.recv_stride;
   float* g = const_cast<float*>(p.diff[rank]);
   const bool zero = p.zero_diff != 0;
 
@@ -98,15 +108,10 @@ __global__ void __launch_bounds__(kPushThreads, 2) fused_sync_sgd_push_kernel(co
         for (int d = 0; d < D; ++d) {
           const int q = peer(rank, 1 + d, N);
           const ShardRange r = shard_range(p.count, N, q);
-          const uint64_t i = vec_elem(r, j), base = r.vec_base << 2;  // slot element 0 <-> global element base
+          const uint64_t i = vec_elem(r, j), base = r.vec_base << 2;
           if (i != ~0ull) {
-            if (BF16) {
-              const uint2 o = pack_bf16x4(v[u][d]);
-              uint16_t* dst = static_cast<uint16_t*>(p.recv[q]) + static_cast<uint64_t>(rank) * slot + (i - base);
-              asm volatile("st.global.v2.u32 [%0], {%1,%2};" ::"l"(dst), "r"(o.x), "r"(o.y) : "memory");
-            } else {
-              st_vec(static_cast<float*>(p.recv[q]) + static_cast<uint64_t>(rank) * slot + (i - base), v[u][d]);
-            }
+            if (BF16) st_vec_u2(recv_slot<uint16_t>(p, q, rank) + (i - base), pack_bf16x4(v[u][d]));
+            else st_vec(recv_slot<float>(p, q, rank) + (i - base), v[u][d]);
           }
         }
       }
@@ -120,13 +125,8 @@ __global__ void __launch_bounds__(kPushThreads, 2) fused_sync_sgd_push_kernel(co
         const uint64_t i = vec_elem(r, j);
         if (i == ~0ull) continue;
         const float4 v = ld_stream(g + i);
-        if (BF16) {
-          const uint2 o = pack_bf16x4(v);
-          uint16_t* dst = static_cast<uint16_t*>(p.recv[q]) + static_cast<uint64_t>(rank) * slot + (i - base);
-          asm volatile("st.global.v2.u32 [%0], {%1,%2};" ::"l"(dst), "r"(o.x), "r"(o.y) : "memory");
-        } else {
-          st_vec(static_cast<float*>(p.recv[q]) + static_cast<uint64_t>(rank) * slot + (i - base), v);
-        }
+        if (BF16) st_vec_u2(recv_slot<uint16_t>(p, q, rank) + (i - base), pack_bf16x4(v));
+        else st_vec(recv_slot<float>(p, q, rank) + (i - base), v);
       }
     }
   }
@@ -137,8 +137,8 @@ __global__ void __launch_bounds__(kPushThreads, 2) fused_sync_sgd_push_kernel(co
       const uint64_t base = r.vec_base << 2;
       const uint64_t i = edge_element(r, threadIdx.x);
       if (i != ~0ull) {
-        if (BF16) (static_cast<uint16_t*>(p.recv[q]) + static_cast<uint64_t>(rank) * slot)[i - base] = float_to_bf16_bits(g[i]);
-        else (static_cast<float*>(p.recv[q]) + static_cast<uint64_t>(rank) * slot)[i - base] = g[i];
+        if (BF16) recv_slot<uint16_t>(p, q, rank)[i - base] = float_to_bf16_bits(g[i]);
+        else recv_slot<float>(p, q, rank)[i - base] = g[i];
       }
     }
   }
@@ -153,6 +153,7 @@ __global__ void __launch_bounds__(kPushThreads, 2) fused_sync_sgd_push_kernel(co
   if (tracer) p.trace[2] = globaltimer_ns();
 
   // ---- phase 2: reduce (local), update, push the new weights ----------------
+  // inline, not seg_cursor(): rebuilding the pointers here costs spills, e.g. <3,true> 0 -> 12 B, <6,false> 68 -> 84 B
   SegCursor cur;
   cur.end = seg_in_smem ? s_end : p.seg_end;
   cur.lr_mult = seg_in_smem ? s_lr : p.seg_lr_mult;
@@ -179,62 +180,31 @@ __global__ void __launch_bounds__(kPushThreads, 2) fused_sync_sgd_push_kernel(co
       if (N > 0) {
 #pragma unroll
         for (int k = 1; k < M; ++k) {  // all N-1 slot loads in flight together (local memory)
-          int src = rank + k;
-          if (src >= M) src -= M;
-          if (BF16)
-            x[k] = unpack_bf16x4(ld_stream_u2(static_cast<const uint16_t*>(p.recv[rank]) + src * slot + (i - base)));
-          else
-            x[k] = ld_stream(static_cast<const float*>(p.recv[rank]) + src * slot + (i - base));
+          const int src = peer(rank, k, M);
+          if (BF16) x[k] = unpack_bf16x4(ld_stream_u2(recv_slot<const uint16_t>(p, rank, src) + (i - base)));
+          else x[k] = ld_stream(recv_slot<const float>(p, rank, src) + (i - base));
         }
       }
       float4 w = *reinterpret_cast<const float4*>(wl + i);
       float4 h = *reinterpret_cast<const float4*>(hl + i);
-      if (BF16) {
-        x[0].x = round_bf16(x[0].x); x[0].y = round_bf16(x[0].y);
-        x[0].z = round_bf16(x[0].z); x[0].w = round_bf16(x[0].w);
-      }
-      float4 acc = make_float4(__fmul_rn(inv, x[0].x), __fmul_rn(inv, x[0].y), __fmul_rn(inv, x[0].z),
-                               __fmul_rn(inv, x[0].w));
+      if (BF16) x[0] = round_bf16x4(x[0]);
+      float4 acc = scaled(inv, x[0]);
       if (N > 0) {
 #pragma unroll
-        for (int k = 1; k < M; ++k) {
-          acc.x = __fadd_rn(__fmul_rn(inv, x[k].x), acc.x);
-          acc.y = __fadd_rn(__fmul_rn(inv, x[k].y), acc.y);
-          acc.z = __fadd_rn(__fmul_rn(inv, x[k].z), acc.z);
-          acc.w = __fadd_rn(__fmul_rn(inv, x[k].w), acc.w);
-        }
+        for (int k = 1; k < M; ++k) add_scaled(acc, inv, x[k]);
       } else {
         for (int k = 1; k < world; ++k) {
-          int src = rank + k;
-          if (src >= world) src -= world;
+          const int src = peer(rank, k, world);
           float4 y;
-          if (BF16)
-            y = unpack_bf16x4(ld_stream_u2(static_cast<const uint16_t*>(p.recv[rank]) + src * slot + (i - base)));
-          else
-            y = ld_stream(static_cast<const float*>(p.recv[rank]) + src * slot + (i - base));
-          acc.x = __fadd_rn(__fmul_rn(inv, y.x), acc.x);
-          acc.y = __fadd_rn(__fmul_rn(inv, y.y), acc.y);
-          acc.z = __fadd_rn(__fmul_rn(inv, y.z), acc.z);
-          acc.w = __fadd_rn(__fmul_rn(inv, y.w), acc.w);
+          if (BF16) y = unpack_bf16x4(ld_stream_u2(recv_slot<const uint16_t>(p, rank, src) + (i - base)));
+          else y = ld_stream(recv_slot<const float>(p, rank, src) + (i - base));
+          add_scaled(acc, inv, y);
         }
       }
       sgd_vec(p, cur, i, acc, w, h);
       *reinterpret_cast<float4*>(hl + i) = h;
       *reinterpret_cast<float4*>(wl + i) = w;
-      if (N > 0) {
-#pragma unroll
-        for (int k = 1; k < M; ++k) {
-          int dst = rank + k;
-          if (dst >= M) dst -= M;
-          st_vec(p.data[dst] + i, w);
-        }
-      } else {
-        for (int k = 1; k < world; ++k) {
-          int dst = rank + k;
-          if (dst >= world) dst -= world;
-          st_vec(p.data[dst] + i, w);
-        }
-      }
+      for_peers<N>(world, [&](int k) { st_vec(p.data[peer(rank, k, world)] + i, w); });
     }
     if (blockIdx.x == 0) {  // scalar head / tail of my shard
       const uint64_t i = edge_element(r, threadIdx.x);
@@ -242,8 +212,8 @@ __global__ void __launch_bounds__(kPushThreads, 2) fused_sync_sgd_push_kernel(co
         float acc = scaled(inv, BF16 ? round_bf16(g[i]) : g[i]);
         for (int k = 1; k < world; ++k) {
           const int src = peer(rank, k, world);
-          const float y = BF16 ? bf16_bits_to_float(static_cast<const uint16_t*>(p.recv[rank])[src * slot + (i - base)])
-                               : static_cast<const float*>(p.recv[rank])[src * slot + (i - base)];
+          const float y = BF16 ? bf16_bits_to_float(recv_slot<const uint16_t>(p, rank, src)[i - base])
+                               : recv_slot<const float>(p, rank, src)[i - base];
           add_scaled(acc, inv, y);
         }
         store_peers(p, world, i, sgd_scalar(p, cur, i, acc, wl, hl));

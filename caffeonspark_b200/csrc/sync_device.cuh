@@ -1,14 +1,16 @@
 // sync_device.cuh -- building blocks shared by the five variants of the fused
 // sync kernel (fused_sync_sgd.cu: LDG/STG pull, _tma.cu: cp.async.bulk pull,
 // _push.cu: stores only, _ll.cu: flag-in-data words, _nvls.cu: multimem):
-// PTX wrappers, bf16 pack / unpack / round, the ring order of the peers and the
-// scale-then-sum step of the reduction, the per-CTA cross-GPU barrier, the
-// shard/vector partition and its scalar head / tail, zeroing of diff_, the blob
-// (segment) cursor and its shared-memory copy, the SGD update of a vector and of
-// a scalar element in the reference's operation order, and the host side of
-// the launchers (argument check, SM count, world-size dispatch).  Not every
-// kernel uses every helper: where a helper changed a kernel's register
-// allocation, the kernel keeps its inline form (see DESIGN.md §3).
+// PTX wrappers, bf16 pack / unpack / round, the ring order of the peers (peer)
+// and the scale-then-sum step of the reduction (scaled / add_scaled, and
+// reduce_scalar over every rank's diff_ or bf16 wire), the per-CTA cross-GPU
+// barrier, the shard bounds (chunk), the shard/vector partition and its scalar
+// head / tail, zeroing of diff_, the blob (segment) cursor and its shared-memory
+// copy, the SGD update of a vector and of a scalar element in the reference's
+// operation order, the all-gather of a scalar weight, and the host side of the
+// launchers (argument check, SM count, world-size dispatch).  Every kernel
+// uses these except in the few places listed in DESIGN.md §3, where the helper
+// changed the kernel's spills or static instruction counts.
 #ifndef COS_SYNC_DEVICE_CUH_
 #define COS_SYNC_DEVICE_CUH_
 
@@ -227,11 +229,16 @@ __device__ __forceinline__ uint64_t vec_elem(const ShardRange& r, uint64_t a) {
   return (a >= r.off && a - r.off < r.nvec) ? ((r.vec_base + a) << 2) : ~0ull;
 }
 
+// First element of shard s; shard s is [chunk(count, world, s), chunk(count, world, s + 1)).
 // socket_sync_cpu.cpp:46-54 chunk(): multiply first, then divide, in 64 bit.
+__device__ __forceinline__ uint64_t chunk(uint64_t count, int world, uint64_t s) {
+  return s * count / static_cast<uint64_t>(world);
+}
+
 __device__ __forceinline__ ShardRange shard_range(uint64_t count, int world, int s) {
   ShardRange r;
-  r.lo = static_cast<uint64_t>(s) * count / static_cast<uint64_t>(world);
-  r.hi = (static_cast<uint64_t>(s) + 1) * count / static_cast<uint64_t>(world);
+  r.lo = chunk(count, world, s);
+  r.hi = chunk(count, world, s + 1ull);
   uint64_t vlo = (r.lo + 3) >> 2, vhi = r.hi >> 2;
   if (vhi > vlo) {
     r.vec_lo = vlo;
@@ -306,20 +313,27 @@ struct SegCursor {
   }
 };
 
-// Copies the segment table to shared memory at smem when it has at most max_seg entries (otherwise the cursor
-// reads global memory) and returns a cursor over it.  The CTA must __syncthreads() before the first seek.
-__device__ __forceinline__ SegCursor load_seg_table(const SyncParams& p, unsigned char* smem, int max_seg) {
+// The segment table lives in shared memory at smem when it has at most max_seg entries; otherwise the cursor reads
+// global memory.  copy_seg_table copies it there; the CTA must __syncthreads() before the first seek of a cursor
+// from seg_cursor.  A kernel short of registers builds the cursor where it first needs it, not at kernel entry.
+__device__ __forceinline__ void copy_seg_table(const SyncParams& p, unsigned char* smem, int max_seg) {
   uint64_t* s_end = reinterpret_cast<uint64_t*>(smem);
   float* s_lr = reinterpret_cast<float*>(s_end + p.nseg);
   float* s_dm = s_lr + p.nseg;
-  const bool in_smem = p.nseg <= max_seg;
-  if (in_smem) {
+  if (p.nseg <= max_seg) {
     for (int k = threadIdx.x; k < p.nseg; k += blockDim.x) {
       s_end[k] = p.seg_end[k];
       s_lr[k] = p.seg_lr_mult[k];
       s_dm[k] = p.seg_decay_mult[k];
     }
   }
+}
+
+__device__ __forceinline__ SegCursor seg_cursor(const SyncParams& p, unsigned char* smem, int max_seg) {
+  uint64_t* s_end = reinterpret_cast<uint64_t*>(smem);
+  float* s_lr = reinterpret_cast<float*>(s_end + p.nseg);
+  float* s_dm = s_lr + p.nseg;
+  const bool in_smem = p.nseg <= max_seg;
   SegCursor c;
   c.end = in_smem ? s_end : p.seg_end;
   c.lr_mult = in_smem ? s_lr : p.seg_lr_mult;
@@ -327,6 +341,11 @@ __device__ __forceinline__ SegCursor load_seg_table(const SyncParams& p, unsigne
   c.nseg = p.nseg;
   c.k = 0;
   return c;
+}
+
+__device__ __forceinline__ SegCursor load_seg_table(const SyncParams& p, unsigned char* smem, int max_seg) {
+  copy_seg_table(p, smem, max_seg);
+  return seg_cursor(p, smem, max_seg);
 }
 
 // Regularize + ComputeUpdateValue + Blob::Update for one element, in the
@@ -398,6 +417,21 @@ __device__ __forceinline__ float sgd_scalar(const SyncParams& p, SegCursor c, ui
   hl[i] = h;
   wl[i] = w;
   return w;
+}
+
+// Scalar element i of shard s summed over every rank's diff_ (or bf16 wire) in the reference's order s, s+1, ...
+// (mod N), each term scaled by 1/N first: the scalar head / tail of the pull kernels, and every element when the
+// world size is known at run time only.
+template <bool BF16>
+__device__ __forceinline__ float reduce_scalar(const SyncParams& p, int s, uint64_t i) {
+  float acc = 0.f;
+  for (int j = 0; j < p.world; ++j) {
+    const int src = peer(s, j, p.world);
+    const float x = BF16 ? bf16_bits_to_float(p.wire[src][i]) : p.diff[src][i];
+    if (j == 0) acc = scaled(p.inv_scale, x);
+    else add_scaled(acc, p.inv_scale, x);
+  }
+  return acc;
 }
 
 // the all-gather of one scalar weight: element i of every peer's data_
