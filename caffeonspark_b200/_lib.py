@@ -33,7 +33,8 @@ class cos_solver_desc(ctypes.Structure):
                 ("nstepvalues", ctypes.c_int), ("max_iter", ctypes.c_int), ("momentum", ctypes.c_float),
                 ("weight_decay", ctypes.c_float), ("test_iter", ctypes.c_int), ("test_interval", ctypes.c_int),
                 ("snapshot_prefix", ctypes.c_char_p), ("grad_dtype", ctypes.c_int), ("init_iter", ctypes.c_int),
-                ("regularization_l1", ctypes.c_int)]
+                ("regularization_l1", ctypes.c_int), ("type", ctypes.c_char_p), ("delta", ctypes.c_float),
+                ("rms_decay", ctypes.c_float)]
 
 
 FORWARD_BACKWARD_FN = ctypes.CFUNCTYPE(ctypes.c_int, ctypes.c_void_p, ctypes.c_int, ctypes.POINTER(cos_blob),
@@ -77,6 +78,7 @@ SYMBOLS = [
     ("cos_net_data", _vp, [_vp, _i]),
     ("cos_net_diff", _vp, [_vp, _i]),
     ("cos_net_history", _vp, [_vp, _i]),
+    ("cos_net_update_history", _vp, [_vp, _i]),
     ("cos_net_param_count", _i64, [_vp]),
     ("cos_net_shard", _i, [_vp, _i, _c.POINTER(_u64), _c.POINTER(_u64)]),
     ("cos_net_iter", _i, [_vp]),

@@ -45,7 +45,7 @@ class SolverDesc:
     def __init__(self, counts, lr_mult=None, decay_mult=None, lr_policy="fixed", base_lr=0.01, gamma=0.0, power=0.0,
                  stepsize=1, stepvalues=(), max_iter=0, momentum=0.0, weight_decay=0.0, test_iter=0,
                  test_interval=0, snapshot_prefix="", grad_dtype="fp32", init_iter=0, batch_size=0,
-                 regularization_type="L2"):
+                 regularization_type="L2", type="SGD", delta=1e-8, rms_decay=0.0):
         self.counts = [int(c) for c in counts]
         self.lr_mult = [float(x) for x in (lr_mult if lr_mult is not None else [1.0] * len(self.counts))]
         self.decay_mult = [float(x) for x in (decay_mult if decay_mult is not None else [1.0] * len(self.counts))]
@@ -55,6 +55,7 @@ class SolverDesc:
         self.test_iter, self.test_interval, self.snapshot_prefix = test_iter, test_interval, snapshot_prefix
         self.grad_dtype, self.init_iter, self.batch_size = grad_dtype, init_iter, batch_size
         self.regularization_type = regularization_type
+        self.type, self.delta, self.rms_decay = type, delta, rms_decay  # SolverParameter.type / delta / rms_decay
 
     @property
     def param_count(self):
@@ -73,7 +74,7 @@ class SolverDesc:
                     lr=(ctypes.c_float * max(1, n))(*self.lr_mult),
                     dm=(ctypes.c_float * max(1, n))(*self.decay_mult),
                     sv=(ctypes.c_int * max(1, len(self.stepvalues)))(*self.stepvalues),
-                    pol=self.lr_policy.encode(), pre=self.snapshot_prefix.encode())
+                    pol=self.lr_policy.encode(), pre=self.snapshot_prefix.encode(), typ=self.type.encode())
         d = cos_solver_desc()
         d.nblobs, d.counts, d.lr_mult, d.decay_mult = n, keep["counts"], keep["lr"], keep["dm"]
         d.lr_policy, d.base_lr, d.gamma, d.power = keep["pol"], self.base_lr, self.gamma, self.power
@@ -83,6 +84,7 @@ class SolverDesc:
         d.grad_dtype = 1 if self.grad_dtype == "bf16" else 0
         d.init_iter = int(self.init_iter)
         d.regularization_l1 = 1 if self.regularization_type == "L1" else 0
+        d.type, d.delta, d.rms_decay = keep["typ"], self.delta, self.rms_decay
         return d, keep
 
 
@@ -102,7 +104,8 @@ def parse_solver(solver_conf_file):
                       gamma=d.gamma, power=d.power, stepsize=d.stepsize, stepvalues=list(sv[:d.nstepvalues]),
                       max_iter=d.max_iter, momentum=d.momentum, weight_decay=d.weight_decay, test_iter=d.test_iter,
                       test_interval=d.test_interval, snapshot_prefix=pre.value.decode(), batch_size=bs.value,
-                      regularization_type="L1" if d.regularization_l1 else "L2")
+                      regularization_type="L1" if d.regularization_l1 else "L2", type=d.type.decode(), delta=d.delta,
+                      rms_decay=d.rms_decay)
 
 
 def read_caffemodel_blob(path, layer_name, blob_index=0):
@@ -295,6 +298,9 @@ class CaffeNet:
     def history_ptr(self, solver_index=0):
         return self._L.cos_net_history(self._h, solver_index)
 
+    def update_history_ptr(self, solver_index=0):
+        return self._L.cos_net_update_history(self._h, solver_index)
+
     def _torch_view(self, ptr, solver_index=0):
         import torch
         return torch.as_tensor(_DevArray(ptr, self.param_count()), device=f"cuda:{self.deviceID(solver_index)}")
@@ -308,6 +314,11 @@ class CaffeNet:
 
     def history(self, solver_index=0):
         return self._torch_view(self.history_ptr(solver_index), solver_index)
+
+    def update_history(self, solver_index=0):
+        """AdaDelta's second history (history of updates) as a torch view; None for the other solvers."""
+        ptr = self.update_history_ptr(solver_index)
+        return self._torch_view(ptr, solver_index) if ptr else None
 
     def global_rank(self, solver_index=0):
         """Rank of local solver `solver_index` in the collective of cluster_size x num_local_devices ranks."""

@@ -82,6 +82,7 @@ CaffeNet::CaffeNet(const SolverSpec& spec, int cluster_size, int node_rank, bool
     : spec_(spec), world_(cluster_size), rank_(node_rank), is_training_(is_training) {
   count_ = spec_.param_count();
   iter_ = spec_.init_iter;
+  solver_ = solver_type_id(spec_.type);  // validated by the parser / cos_net_allocate_desc
   if (const char* t = getenv("COS_BARRIER_TIMEOUT_MS")) opt_timeout_ms_ = atoll(t);
 }
 
@@ -151,7 +152,7 @@ bool CaffeNet::allocate_device(int start_device_id, bool peer_mappable, std::str
     return false;
   }
 
-  // arena = [flags | data_ | diff_ | history | bf16 wire]
+  // arena = [flags | data_ | diff_ | history | AdaDelta's second history | bf16 wire]
   const size_t fbytes = static_cast<size_t>(count_) * sizeof(float);
   size_t off = align_up(kFlagBytes, 4096);
   off_data_ = off;
@@ -160,6 +161,8 @@ bool CaffeNet::allocate_device(int start_device_id, bool peer_mappable, std::str
   off = align_up(off + fbytes, 4096);
   off_hist_ = off;
   off = align_up(off + fbytes, 4096);
+  off_hist2_ = off;
+  if (solver_ == kSolverAdaDelta) off = align_up(off + fbytes, 4096);
   off_wire_ = off;
   if (spec_.grad_dtype == COS_GRAD_BF16) off = align_up(off + static_cast<size_t>(count_) * 2, 4096);
   off_recv_ = off;
@@ -181,11 +184,13 @@ bool CaffeNet::allocate_device(int start_device_id, bool peer_mappable, std::str
   data_ = reinterpret_cast<float*>(base + off_data_);
   diff_ = reinterpret_cast<float*>(base + off_diff_);
   hist_ = reinterpret_cast<float*>(base + off_hist_);
+  hist2_ = solver_ == kSolverAdaDelta ? reinterpret_cast<float*>(base + off_hist2_) : nullptr;
   wire_ = spec_.grad_dtype == COS_GRAD_BF16 ? reinterpret_cast<uint16_t*>(base + off_wire_) : nullptr;
   peer_data_[rank_] = data_;
   peer_diff_[rank_] = diff_;
   peer_wire_[rank_] = wire_;
   peer_hist_[rank_] = hist_;
+  peer_hist2_[rank_] = hist2_;
   peer_flags_[rank_] = reinterpret_cast<uint32_t*>(base);
   recv_ = recv_stride_ ? static_cast<void*>(base + off_recv_) : nullptr;
   peer_recv_[rank_] = recv_;
@@ -268,23 +273,28 @@ int CaffeNet::resolved_algo() const {
 //   * otherwise push (stores only; the bf16 cast costs no extra pass; measured >= the TMA pull pipeline at
 //     every size on B200), the TMA pull pipeline above push_max_bytes.
 // A forced variant that cannot run the current mode falls back to AUTO's choice.
+// The TMA and NVLS kernels run SGD only: for any other solver the TMA choices become LDG (a forced kernel 1 too)
+// and NVLS is never chosen (a forced kernel 3 falls back to AUTO's choice).
 int CaffeNet::resolved_kernel() const {
   const int algo = resolved_algo();
   const bool fp32 = spec_.grad_dtype == COS_GRAD_FP32;
+  const bool sgd = solver_ == kSolverSGD;
   const int64_t bytes = static_cast<int64_t>(count_ * sizeof(float));
-  const bool nvls_ok = nvls_active_ && fp32 && algo == kModeTwoShot;
+  const int pull = sgd && bytes >= (2 << 20) ? 1 : 0;  // TMA pull pipeline from 2 MiB on, LDG below
+  const bool nvls_ok = sgd && nvls_active_ && fp32 && algo == kModeTwoShot;
   const bool push_ok = world_ > 1 && algo == kModeTwoShot && recv_stride_ > 0;
   const bool ll_ok = world_ > 1 && algo == kModeTwoShot && ll_grad_stride_ > 0;
-  if (opt_kernel_ == 0 || opt_kernel_ == 1) return opt_kernel_;
+  if (opt_kernel_ == 0) return 0;
+  if (opt_kernel_ == 1) return sgd ? 1 : 0;
   if (opt_kernel_ == 2 && push_ok) return 2;
   if (opt_kernel_ == 3 && nvls_ok) return 3;
   if (opt_kernel_ == 4 && ll_ok) return 4;
   if (world_ == 1) return 0;
-  if (algo != kModeTwoShot) return bytes >= (2 << 20) ? 1 : 0;
+  if (algo != kModeTwoShot) return pull;
   if (nvls_ok && (opt_nvls_ == 1 || (world_ >= kNvlsAutoMinWorld && bytes >= opt_nvls_min_bytes_))) return 3;
   if (ll_ok && bytes < opt_ll_max_bytes_) return 4;
   if (push_ok && (!fp32 || bytes < opt_push_max_bytes_)) return 2;
-  return bytes >= (2 << 20) ? 1 : 0;
+  return pull;
 }
 
 float CaffeNet::current_rate() {
@@ -333,6 +343,19 @@ bool CaffeNet::launch(int mode, cudaStream_t stream, std::string* err) {
   p.timeout_ns = static_cast<unsigned long long>(opt_timeout_ms_) * 1000000ull;
   p.status = status_;
   p.trace = opt_trace_ ? reinterpret_cast<unsigned long long*>(status_) + 2 : nullptr;
+  // the solver's constants in float, as the reference's Dtype expressions compute them
+  const float m = spec_.momentum;
+  p.solver = solver_;
+  p.hist2 = hist2_;
+  p.delta = spec_.delta;
+  if (solver_ == kSolverRMSProp) {  // rmsprop_solver.cpp:31-33: axpby(1 - rms_decay, u, rms_decay, h)
+    p.momentum = spec_.rms_decay;
+    p.one_minus = 1.0f - spec_.rms_decay;
+  } else {
+    p.one_minus = 1.0f - m;         // adadelta_solver.cpp:41-43: Dtype(1) - momentum
+  }
+  p.one_plus_m = 1.0f + m;          // nesterov_solver.cpp:33-35: Dtype(1) + momentum, -momentum
+  p.neg_m = -m;
   if (mode != kModeAllGather) {
     if (!learning_rate(spec_.lr_policy, spec_.base_lr, spec_.gamma, spec_.power, spec_.stepsize,
                        spec_.stepvalues.empty() ? nullptr : spec_.stepvalues.data(),
@@ -654,32 +677,43 @@ int CaffeNet::snapshot(std::string* err) {
     return -1;
   }
   if (!check_status(err)) return -1;
-  std::vector<float> w(count_), h(count_);
+  // history_ = [h of every blob], for AdaDelta followed by [h2 of every blob] (AdaDeltaPreSolve,
+  // adadelta_solver.cpp:7-17): h and h2 are gathered from their shard owners alike
+  const int nhist = hist2_ ? 2 : 1;
+  std::vector<float> w(count_), h(count_ * nhist);
   cudaError_t e = cudaMemcpy(w.data(), data_, count_ * sizeof(float), cudaMemcpyDeviceToHost);
   const bool sharded_hist = world_ > 1 && resolved_algo() == kModeTwoShot;
-  for (int r = 0; r < world_ && e == cudaSuccess; ++r) {
-    uint64_t offs = 0, size = count_;
-    if (sharded_hist) chunk(count_, world_, r, &offs, &size);
-    else if (r != rank_) continue;
-    const float* src = (sharded_hist ? peer_hist_[r] : hist_);
-    if (!src) {
-      *err = "snapshot: history of rank " + std::to_string(r) + " is not mapped (connect() first)";
-      return -1;
+  for (int q = 0; q < nhist; ++q) {
+    for (int r = 0; r < world_ && e == cudaSuccess; ++r) {
+      uint64_t offs = 0, size = count_;
+      if (sharded_hist) chunk(count_, world_, r, &offs, &size);
+      else if (r != rank_) continue;
+      const float* const* peers = q == 0 ? peer_hist_ : peer_hist2_;
+      const float* src = sharded_hist ? peers[r] : (q == 0 ? hist_ : hist2_);
+      if (!src) {
+        *err = "snapshot: history of rank " + std::to_string(r) + " is not mapped (connect() first)";
+        return -1;
+      }
+      if (size) e = cudaMemcpy(h.data() + q * count_ + offs, src + offs, size * sizeof(float), cudaMemcpyDeviceToHost);
     }
-    if (size) e = cudaMemcpy(h.data() + offs, src + offs, size * sizeof(float), cudaMemcpyDeviceToHost);
   }
   if (e != cudaSuccess) {
     *err = rt_err("snapshot: copy to host", e);
     return -1;
   }
+  std::vector<BlobView> hv = blob_views(h.data());
+  if (hist2_) {
+    std::vector<BlobView> hv2 = blob_views(h.data() + count_);
+    hv.insert(hv.end(), hv2.begin(), hv2.end());
+  }
   const std::string model = snapshot_filename(iter_, false), state = snapshot_filename(iter_, true);
   if (spec_.snapshot_hdf5) {  // solver.cpp:417-418 SnapshotToHDF5 + sgd_solver.cpp:251-252 (csrc/hdf5_io.cpp)
     if (!write_caffemodel_h5(model, blob_views(w.data()), err)) return -1;
-    if (!write_solverstate_h5(state, iter_, current_step_, model, blob_views(h.data()), err)) return -1;
+    if (!write_solverstate_h5(state, iter_, current_step_, model, hv, err)) return -1;
     return iter_;
   }
   if (!write_caffemodel(model, spec_.net_name, blob_views(w.data()), err)) return -1;
-  if (!write_solverstate(state, iter_, current_step_, model, blob_views(h.data()), err)) return -1;
+  if (!write_solverstate(state, iter_, current_step_, model, hv, err)) return -1;
   return iter_;
 }
 
@@ -693,24 +727,29 @@ bool CaffeNet::restore(const std::string& model_file, const std::string& state_f
     std::string learned;
     std::vector<ParsedBlob> hist;
     if (!read_solverstate(state_file, &it, &step, &learned, &hist, err)) return false;
-    if (hist.size() != spec_.counts.size()) {
+    const size_t nblobs = spec_.counts.size(), nhist = hist2_ ? 2 : 1;  // AdaDelta: h of every blob, then h2
+    if (hist.size() != nhist * nblobs) {
       *err = "'" + state_file + "' is not a matching snapshot of this net: " + std::to_string(hist.size()) +
-             " history blobs, the net has " + std::to_string(spec_.counts.size()) + " learnable blobs";
+             " history blobs, the net has " + std::to_string(nblobs) + " learnable blobs" +
+             (hist2_ ? " (AdaDelta keeps two history blobs per learnable blob)" : "");
       return false;
     }
-    std::vector<float> flat(count_, 0.f);
+    std::vector<float> flat(count_ * nhist, 0.f);
     uint64_t off = 0;
     for (size_t k = 0; k < hist.size(); ++k) {
-      if (hist[k].data.size() != static_cast<size_t>(spec_.counts[k])) {
+      const size_t b = k % nblobs;
+      if (b == 0) off = (k / nblobs) * count_;
+      if (hist[k].data.size() != static_cast<size_t>(spec_.counts[b])) {
         *err = "'" + state_file + "' is not a matching snapshot of this net: history blob " + std::to_string(k) +
                " has " + std::to_string(hist[k].data.size()) + " elements, expected " +
-               std::to_string(spec_.counts[k]);
+               std::to_string(spec_.counts[b]);
         return false;
       }
       memcpy(flat.data() + off, hist[k].data.data(), hist[k].data.size() * sizeof(float));
       off += hist[k].data.size();
     }
     COS_RT(cudaMemcpy(hist_, flat.data(), count_ * sizeof(float), cudaMemcpyHostToDevice));
+    if (hist2_) COS_RT(cudaMemcpy(hist2_, flat.data() + count_, count_ * sizeof(float), cudaMemcpyHostToDevice));
     iter_ = it;
     current_step_ = step;
     spec_.init_iter = it;
@@ -881,6 +920,7 @@ bool NvlinkCaffeNet::connect(const std::vector<std::string>& addresses, std::str
     peer_data_[peer] = reinterpret_cast<float*>(base + off_data_);
     peer_diff_[peer] = reinterpret_cast<const float*>(base + off_diff_);
     peer_hist_[peer] = reinterpret_cast<const float*>(base + off_hist_);
+    peer_hist2_[peer] = hist2_ ? reinterpret_cast<const float*>(base + off_hist2_) : nullptr;
     peer_wire_[peer] = wire_ ? reinterpret_cast<uint16_t*>(base + off_wire_) : nullptr;
     peer_recv_[peer] = recv_stride_ ? static_cast<void*>(base + off_recv_) : nullptr;
     peer_llg_[peer] = ll_grad_stride_ ? reinterpret_cast<uint64_t*>(base + off_llg_) : nullptr;
@@ -889,7 +929,8 @@ bool NvlinkCaffeNet::connect(const std::vector<std::string>& addresses, std::str
   connected_ = true;
   // NVLS multicast team: on request, or by default where it pays (N >= 6, message >= nvls_min_bytes, fp32 wire).
   // The decision uses only values that are identical on every rank.
-  const bool want_nvls = opt_nvls_ == 1 || (opt_nvls_ < 0 && world_ >= kNvlsAutoMinWorld && spec_.grad_dtype == COS_GRAD_FP32 &&
+  const bool want_nvls = opt_nvls_ == 1 || (opt_nvls_ < 0 && solver_ == kSolverSGD && world_ >= kNvlsAutoMinWorld &&
+                                            spec_.grad_dtype == COS_GRAD_FP32 &&
                                             static_cast<int64_t>(count_ * sizeof(float)) >= opt_nvls_min_bytes_);
   if (want_nvls) setup_nvls(timeout);
   // everyone has mapped everyone; then the first on_start(): all-gather of the

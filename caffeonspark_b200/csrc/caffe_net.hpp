@@ -74,6 +74,7 @@ class CaffeNet {
   float* data() const { return data_; }
   float* diff() const { return diff_; }
   float* history() const { return hist_; }
+  float* update_history() const { return hist2_; }  // AdaDelta's h2, nullptr for the other solvers
   uint64_t param_count() const { return count_; }
   int cluster_size() const { return world_; }
   int rank() const { return rank_; }
@@ -107,6 +108,7 @@ class CaffeNet {
   // Params<Dtype> (parallel.hpp:22-45): flat buffers, inside the peer-mappable arena
   DeviceArena arena_;
   size_t off_data_ = 0, off_diff_ = 0, off_hist_ = 0, off_wire_ = 0, off_recv_ = 0;
+  size_t off_hist2_ = 0;           // AdaDelta only: second history region right after history
   uint64_t recv_stride_ = 0;       // elements per receive slot of the push kernel (0: no receive region)
   void* recv_ = nullptr;           // [world][recv_stride_] fp32 or bf16: the reference's diff_recv_ scratch, on device
   size_t off_llg_ = 0, off_llw_ = 0;  // LL kernel slots (small nets only): [world][ll_*_stride_] 8-byte words
@@ -116,6 +118,8 @@ class CaffeNet {
   uint16_t* wire_ = nullptr;
   float* hist_ = nullptr;          // SGDSolver::history_ (sgd_solver.cpp:66-78); in the arena so that a
                                    // snapshot on rank 0 can read the owners' shards
+  float* hist2_ = nullptr;         // AdaDelta's history of updates (history_[n + i]), nullptr for the other solvers
+  int solver_ = kSolverSGD;        // SolverType of spec_.type
   uint64_t* seg_end_ = nullptr;    // device copies of the blob table
   float* seg_lr_ = nullptr;
   float* seg_dm_ = nullptr;
@@ -129,6 +133,7 @@ class CaffeNet {
   const float* peer_diff_[kMaxRanks] = {};
   uint16_t* peer_wire_[kMaxRanks] = {};
   const float* peer_hist_[kMaxRanks] = {};
+  const float* peer_hist2_[kMaxRanks] = {};
   uint32_t* peer_flags_[kMaxRanks] = {};
   void* peer_recv_[kMaxRanks] = {};
   uint64_t* peer_llg_[kMaxRanks] = {};

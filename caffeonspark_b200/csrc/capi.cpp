@@ -79,6 +79,10 @@ bool spec_from_desc(const cos_solver_desc* d, SolverSpec* s, std::string* err) {
   s->grad_dtype = d->grad_dtype;
   s->init_iter = d->init_iter;
   s->regularization_type = d->regularization_l1 ? "L1" : "L2";
+  s->type = d->type ? d->type : "SGD";
+  s->delta = d->delta;
+  s->rms_decay = d->rms_decay;
+  if (!cosb::validate_solver(*s, err)) return false;
   float r;
   int step = 0;
   if (!cosb::learning_rate(s->lr_policy, s->base_lr, s->gamma, s->power, s->stepsize,
@@ -283,6 +287,10 @@ float* cos_net_diff(cos_net* net, int solver_index) {
 float* cos_net_history(cos_net* net, int solver_index) {
   CaffeNet* r = R(net, solver_index);
   return r ? r->history() : nullptr;
+}
+float* cos_net_update_history(cos_net* net, int solver_index) {
+  CaffeNet* r = R(net, solver_index);
+  return r ? r->update_history() : nullptr;
 }
 int64_t cos_net_param_count(cos_net* net) { return net ? static_cast<int64_t>(R(net, 0)->param_count()) : -1; }
 
@@ -620,6 +628,9 @@ int cos_parse_solver(const char* solver_conf_file, cos_solver_desc* desc, int64_
     desc->momentum = s.momentum;
     desc->weight_decay = s.weight_decay;
     desc->regularization_l1 = s.regularization_type == "L1" ? 1 : 0;
+    desc->type = cosb::solver_type_name(cosb::solver_type_id(s.type));
+    desc->delta = s.delta;
+    desc->rms_decay = s.rms_decay;
     desc->test_iter = s.test_iter;
     desc->test_interval = s.test_interval;
     if (batch_size) *batch_size = s.batch_size;

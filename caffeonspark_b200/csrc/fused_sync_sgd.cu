@@ -67,9 +67,9 @@ __device__ __forceinline__ float4 reduce_vec_any(const SyncParams& p, int s, uin
 
 // ------------------------------------------------------------- the kernel
 
-// N = compile-time world size (0 = runtime world, any size up to kMaxRanks).
+// N = compile-time world size (0 = runtime world, any size up to kMaxRanks), S = SolverType.
 // (The in-switch NVLS variant lives in fused_sync_sgd_nvls.cu.)
-template <int N, bool BF16>
+template <int N, bool BF16, int S = kSolverSGD>
 __global__ void __launch_bounds__(kDefaultThreads, 2) fused_sync_sgd_kernel(const SyncParams p) {
   extern __shared__ unsigned char smem_raw[];
   __shared__ int s_abort;
@@ -143,7 +143,7 @@ __global__ void __launch_bounds__(kDefaultThreads, 2) fused_sync_sgd_kernel(cons
         } else {
           g = reduce_vec_any<N, BF16>(p, s, i);
         }
-        sgd_vec(p, cur, i, g, w, h);
+        update_vec<S>(p, cur, i, g, w, h);
         *reinterpret_cast<float4*>(hl + i) = h;
         *reinterpret_cast<float4*>(wl + i) = w;
         if (push) for_peers<N>(world, [&](int q) { st_vec(p.data[peer(rank, q, world)] + i, w); });
@@ -153,7 +153,7 @@ __global__ void __launch_bounds__(kDefaultThreads, 2) fused_sync_sgd_kernel(cons
         if (i != ~0ull) {
           float g = (p.mode == kModeLocal) ? p.diff[rank][i] : reduce_scalar<BF16>(p, s, i);
           if (BF16 && p.mode == kModeLocal) g = round_bf16(g);
-          const float w = sgd_scalar(p, cur, i, g, wl, hl);
+          const float w = update_scalar<S>(p, cur, i, g, wl, hl);
           if (push) store_peers(p, world, i, w);
         }
       }
@@ -229,10 +229,12 @@ cudaError_t launch_fused_sync_sgd(const SyncParams& p, int grid, int block, cuda
   if (static_cast<uint64_t>(grid) > need) grid = static_cast<int>(need);
   const size_t smem = seg_smem_bytes(p, kMaxSegSmem);
   const int n = (p.mode == kModeLocal || p.mode == kModeAllGather) ? 0 : p.world;
-  return dispatch_world(n, [&](auto N) {
-    if (p.grad_bf16) fused_sync_sgd_kernel<N, true><<<grid, block, smem, stream>>>(p);
-    else fused_sync_sgd_kernel<N, false><<<grid, block, smem, stream>>>(p);
-    return cudaGetLastError();
+  return dispatch_solver(p.solver, [&](auto S) {
+    return dispatch_world(n, [&](auto N) {
+      if (p.grad_bf16) fused_sync_sgd_kernel<N, true, S><<<grid, block, smem, stream>>>(p);
+      else fused_sync_sgd_kernel<N, false, S><<<grid, block, smem, stream>>>(p);
+      return cudaGetLastError();
+    });
   });
 }
 

@@ -26,6 +26,15 @@ enum SyncMode : int {
   kModeAllGather = 3,  // on_start() alone: push owned weight shard to peers
 };
 
+// Solver of the update half (SolverParameter.type).  The kernels are templates on it; TMA and NVLS run SGD only.
+enum SolverType : int {
+  kSolverSGD = 0,
+  kSolverNesterov = 1,
+  kSolverAdaGrad = 2,
+  kSolverRMSProp = 3,
+  kSolverAdaDelta = 4,
+};
+
 struct SyncParams {
   int world;
   int rank;
@@ -54,7 +63,7 @@ struct SyncParams {
   const float* seg_lr_mult;         // [nseg]
   const float* seg_decay_mult;      // [nseg]
   float rate;                       // GetLearningRate() of this iteration
-  float momentum;
+  float momentum;                   // the factor h is scaled by: momentum, or rms_decay for RMSProp
   float weight_decay;
   float inv_scale;                  // (float)(1.0 / solver_count)
   uint32_t epoch;                   // barrier epoch of this launch
@@ -62,8 +71,17 @@ struct SyncParams {
   int* status;                      // local device word: 0 ok, else error code
   unsigned long long* trace;        // optional: 13 x %globaltimer of CTA 0: [0..4] phase boundaries, [5..8] / [9..12]
                                     // inside barrier A / B (entered, release fence done, flag arrived, acquire done)
+  // Solver fields, appended so that every field above keeps its offset in the kernel parameter block.  The host
+  // derives the constants in float, as the reference's Dtype arithmetic does; the device never re-derives them.
+  int solver;                       // SolverType
+  float* hist2;                     // AdaDelta: local history of updates (history_[n + i]); null otherwise
+  float delta;                      // SolverParameter.delta (AdaGrad, RMSProp, AdaDelta)
+  float one_minus;                  // 1 - momentum (AdaDelta) or 1 - rms_decay (RMSProp)
+  float one_plus_m;                 // 1 + momentum (Nesterov)
+  float neg_m;                      // -momentum (Nesterov)
 };
 
+// The LDG, push and LL launchers run every SolverType; TMA and NVLS return cudaErrorInvalidValue for p.solver != SGD.
 // Launches the vector (LDG/STG) kernel.  grid/block 0 = defaults.
 cudaError_t launch_fused_sync_sgd(const SyncParams& p, int grid, int block, cudaStream_t stream);
 // Launches the TMA (cp.async.bulk) pipelined variant of the same computation.

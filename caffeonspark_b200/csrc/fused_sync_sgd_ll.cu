@@ -125,8 +125,8 @@ __device__ __forceinline__ uint64_t edge_index(const ShardRange& r, uint64_t e) 
   return e < r.head_end ? e - r.lo : 4 + (e - r.tail_begin);
 }
 
-// N = compile-time world size, 2..8 (the N-1 polled slots live in registers)
-template <int N, bool BF16>
+// N = compile-time world size, 2..8 (the N-1 polled slots live in registers); S = SolverType
+template <int N, bool BF16, int S = kSolverSGD>
 __global__ void __launch_bounds__(kLLThreads, 1) fused_sync_sgd_ll_kernel(const SyncParams p) {
   extern __shared__ unsigned char smem_raw[];
   __shared__ int s_abort;
@@ -241,7 +241,7 @@ __global__ void __launch_bounds__(kLLThreads, 1) fused_sync_sgd_ll_kernel(const 
         add_scaled(acc, inv, y);
       }
       if (!alive) break;
-      sgd_vec(p, cur, i, acc, w, h);
+      update_vec<S>(p, cur, i, acc, w, h);
       *reinterpret_cast<float4*>(hl + i) = h;
       *reinterpret_cast<float4*>(wl + i) = w;
       const uint64_t wa = ll_word(__float_as_uint(w.x), flag), wb = ll_word(__float_as_uint(w.y), flag);
@@ -264,7 +264,7 @@ __global__ void __launch_bounds__(kLLThreads, 1) fused_sync_sgd_ll_kernel(const 
           if (alive) add_scaled(acc, inv, __uint_as_float(u));
         }
         if (alive) {
-          const float w = sgd_scalar(p, cur, e, acc, wl, hl);
+          const float w = update_scalar<S>(p, cur, e, acc, wl, hl);
           for (int k = 1; k < world; ++k) {
             const int dst = peer(rank, k, world);
             st_ll1(p.ll_weight[dst] + static_cast<uint64_t>(rank) * wslot + wedge + edge_index(r, e),
@@ -355,14 +355,16 @@ cudaError_t launch_fused_sync_sgd_ll(const SyncParams& p, int grid, int block, i
   }
   if (grid > cap) grid = cap;
   const size_t smem = seg_smem_bytes(p, kLLMaxSeg);
-  return dispatch_world(p.world, [&](auto N) {
-    if constexpr (decltype(N)::value == 0) {
-      return cudaErrorInvalidValue;  // world sizes 9..16 use the barrier-based kernels
-    } else {
-      if (p.grad_bf16) fused_sync_sgd_ll_kernel<N, true><<<grid, block, smem, stream>>>(p);
-      else fused_sync_sgd_ll_kernel<N, false><<<grid, block, smem, stream>>>(p);
-      return cudaGetLastError();
-    }
+  return dispatch_solver(p.solver, [&](auto S) {
+    return dispatch_world(p.world, [&](auto N) {
+      if constexpr (decltype(N)::value == 0) {
+        return cudaErrorInvalidValue;  // world sizes 9..16 use the barrier-based kernels
+      } else {
+        if (p.grad_bf16) fused_sync_sgd_ll_kernel<N, true, S><<<grid, block, smem, stream>>>(p);
+        else fused_sync_sgd_ll_kernel<N, false, S><<<grid, block, smem, stream>>>(p);
+        return cudaGetLastError();
+      }
+    });
   });
 }
 

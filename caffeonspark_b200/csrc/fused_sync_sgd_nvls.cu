@@ -232,6 +232,7 @@ cudaError_t launch_share(const SyncParams& p, int grid, size_t smem, cudaStream_
 
 cudaError_t launch_fused_sync_sgd_nvls(const SyncParams& p, int grid, cudaStream_t stream) {
   if (!check_world(p, 2)) return cudaErrorInvalidValue;
+  if (p.solver != kSolverSGD) return cudaErrorInvalidValue;  // SGD only: the routing never sends another solver here
   if (p.mode != kModeTwoShot || p.grad_bf16 || !p.mc_data || !p.mc_diff) return cudaErrorInvalidValue;
   if (grid <= 0) grid = sm_count(-1);  // __launch_bounds__(512, 1): one resident CTA per SM
   if (grid > kMaxCtas) grid = kMaxCtas;

@@ -53,8 +53,8 @@ __device__ __forceinline__ T* recv_slot(const SyncParams& p, int q, int src) {
   return static_cast<T*>(p.recv[q]) + static_cast<uint64_t>(src) * p.recv_stride;
 }
 
-// N = compile-time world size (2..8), 0 = run-time world (<= kMaxRanks)
-template <int N, bool BF16>
+// N = compile-time world size (2..8), 0 = run-time world (<= kMaxRanks); S = SolverType
+template <int N, bool BF16, int S = kSolverSGD>
 __global__ void __launch_bounds__(kPushThreads, 2) fused_sync_sgd_push_kernel(const SyncParams p) {
   extern __shared__ unsigned char smem_raw[];
   __shared__ int s_abort;
@@ -201,7 +201,7 @@ __global__ void __launch_bounds__(kPushThreads, 2) fused_sync_sgd_push_kernel(co
           add_scaled(acc, inv, y);
         }
       }
-      sgd_vec(p, cur, i, acc, w, h);
+      update_vec<S>(p, cur, i, acc, w, h);
       *reinterpret_cast<float4*>(hl + i) = h;
       *reinterpret_cast<float4*>(wl + i) = w;
       for_peers<N>(world, [&](int k) { st_vec(p.data[peer(rank, k, world)] + i, w); });
@@ -216,7 +216,7 @@ __global__ void __launch_bounds__(kPushThreads, 2) fused_sync_sgd_push_kernel(co
                                : recv_slot<const float>(p, rank, src)[i - base];
           add_scaled(acc, inv, y);
         }
-        store_peers(p, world, i, sgd_scalar(p, cur, i, acc, wl, hl));
+        store_peers(p, world, i, update_scalar<S>(p, cur, i, acc, wl, hl));
       }
     }
   }
@@ -258,10 +258,12 @@ cudaError_t launch_fused_sync_sgd_push(const SyncParams& p, int grid, int block,
   }
   if (grid > kMaxCtas) grid = kMaxCtas;
   const size_t smem = seg_smem_bytes(p, kPushMaxSeg);
-  return dispatch_world(p.world, [&](auto N) {
-    if (p.grad_bf16) fused_sync_sgd_push_kernel<N, true><<<grid, block, smem, stream>>>(p);
-    else fused_sync_sgd_push_kernel<N, false><<<grid, block, smem, stream>>>(p);
-    return cudaGetLastError();
+  return dispatch_solver(p.solver, [&](auto S) {
+    return dispatch_world(p.world, [&](auto N) {
+      if (p.grad_bf16) fused_sync_sgd_push_kernel<N, true, S><<<grid, block, smem, stream>>>(p);
+      else fused_sync_sgd_push_kernel<N, false, S><<<grid, block, smem, stream>>>(p);
+      return cudaGetLastError();
+    });
   });
 }
 

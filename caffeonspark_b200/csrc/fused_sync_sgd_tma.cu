@@ -369,6 +369,7 @@ fused_sync_sgd_tma_kernel(const SyncParams p, const int tile_elems) {
 
 cudaError_t launch_fused_sync_sgd_tma(const SyncParams& p, int grid, cudaStream_t stream) {
   if (!check_world(p, 1) || p.mode == kModeAllGather) return cudaErrorInvalidValue;
+  if (p.solver != kSolverSGD) return cudaErrorInvalidValue;  // SGD only: the routing never sends another solver here
   if (grid <= 0) grid = sm_count(-1);  // persistent: one CTA per SM
   if (grid > kMaxCtas) grid = kMaxCtas;
   const int nsrc = p.mode == kModeLocal ? 1 : p.world;

@@ -1,6 +1,8 @@
 // solver_spec.cpp -- see solver_spec.hpp.
 #include "solver_spec.hpp"
 
+#include "fused_sync_sgd.hpp"
+
 #include <math.h>
 #include <stdlib.h>
 
@@ -60,6 +62,37 @@ bool learning_rate(const std::string& policy, float base_lr, float gamma, float 
     *rate = static_cast<float>(static_cast<double>(base_lr) * d);
   } else {
     return false;  // LOG(FATAL) << "Unknown learning rate policy" (:60)
+  }
+  return true;
+}
+
+namespace {
+const char* const kSolverNames[] = {"SGD", "Nesterov", "AdaGrad", "RMSProp", "AdaDelta"};
+const char* const kSolverEnums[] = {"SGD", "NESTEROV", "ADAGRAD", "RMSPROP", "ADADELTA"};  // caffe.proto SolverType
+}  // namespace
+
+const char* solver_type_name(int id) { return id >= 0 && id < 5 ? kSolverNames[id] : nullptr; }
+
+int solver_type_id(const std::string& type) {
+  for (int k = 0; k < 5; ++k)
+    if (type == kSolverNames[k]) return k;
+  return -1;
+}
+
+bool validate_solver(const SolverSpec& spec, std::string* err) {
+  const int id = solver_type_id(spec.type);
+  if (id < 0) {
+    *err = "solver type '" + spec.type +
+           "' is not on the accelerated path (only SGD, Nesterov, AdaGrad, RMSProp and AdaDelta are)";
+    return false;
+  }
+  if ((id == kSolverAdaGrad || id == kSolverRMSProp) && spec.momentum != 0.f) {
+    *err = std::string("Momentum cannot be used with ") + kSolverNames[id] + ".";
+    return false;
+  }
+  if (id == kSolverRMSProp && !(spec.rms_decay >= 0.f && spec.rms_decay < 1.f)) {
+    *err = "rms_decay should lie between 0 and 1.";
+    return false;
   }
   return true;
 }
@@ -496,15 +529,15 @@ bool parse_solver_prototxt(const std::string& solver_path, SolverSpec* spec, std
   spec->solver_mode_gpu = s.str("solver_mode", "GPU") != "CPU";
   spec->snapshot_hdf5 = s.str("snapshot_format", "BINARYPROTO") == "HDF5";
   std::string type = s.str("type", "");
-  if (type.empty()) {
-    std::string st = s.str("solver_type", "SGD");  // deprecated enum field
-    type = st;
+  if (type.empty()) {  // deprecated enum field solver_type (caffe.proto SolverType), upgraded to the type name
+    type = s.str("solver_type", "SGD");
+    for (int k = 0; k < 5; ++k)
+      if (type == kSolverEnums[k]) type = kSolverNames[k];
   }
   spec->type = type;
-  if (spec->type != "SGD") {
-    *err = "solver type '" + spec->type + "' is not on the accelerated path (only SGD with momentum is)";
-    return false;
-  }
+  spec->delta = static_cast<float>(s.num("delta", 1e-8));
+  spec->rms_decay = static_cast<float>(s.num("rms_decay", 0.0));
+  if (!validate_solver(*spec, err)) return false;
   if (spec->regularization_type != "L2" && spec->regularization_type != "L1") {
     *err = "Unknown regularization type: " + spec->regularization_type;  // sgd_solver.cpp:169-171
     return false;

@@ -36,7 +36,9 @@ struct SolverSpec {
   int test_iter = 0, test_interval = 0;
   std::string snapshot_prefix;
   std::string regularization_type = "L2";
-  std::string type = "SGD";
+  std::string type = "SGD";       // SGD | Nesterov | AdaGrad | RMSProp | AdaDelta (canonical spelling)
+  float delta = 1e-8f;             // SolverParameter.delta (caffe.proto: default 1e-8)
+  float rms_decay = 0.f;           // SolverParameter.rms_decay (no default: 0)
   int iter_size = 1;
   float clip_gradients = -1.f;
   bool solver_mode_gpu = true;
@@ -58,6 +60,15 @@ void chunk(uint64_t param_count, int cluster_size, int peer, uint64_t* offs, uin
 bool learning_rate(const std::string& policy, float base_lr, float gamma, float power, int stepsize,
                    const int* stepvalues, int nstepvalues, int max_iter, int iter, int* current_step,
                    float* rate);
+
+// SolverType (fused_sync_sgd.hpp) of a canonical type name, -1 for any other name.
+int solver_type_id(const std::string& type);
+// The canonical name of SolverType `id` (static storage), nullptr for any other value.
+const char* solver_type_name(int id);
+// Checks type, momentum and rms_decay as the reference's solver constructors do (sgd_solvers.hpp:70-100).  Shared
+// by the prototxt parser (which maps the deprecated solver_type enum to the type name first) and
+// cos_net_allocate_desc.
+bool validate_solver(const SolverSpec& spec, std::string* err);
 
 // Parses a solver prototxt and the net it references (net:, train_net: or
 // inline net_param/train_net_param) and fills `spec`.

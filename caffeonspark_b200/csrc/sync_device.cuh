@@ -7,8 +7,10 @@
 // barrier, the shard bounds (chunk), the shard/vector partition and its scalar
 // head / tail, zeroing of diff_, the blob (segment) cursor and its shared-memory
 // copy, the SGD update of a vector and of a scalar element in the reference's
-// operation order, the all-gather of a scalar weight, and the host side of the
-// launchers (argument check, SM count, world-size dispatch).  Every kernel
+// operation order and the same for the Nesterov, AdaGrad, RMSProp and AdaDelta
+// solvers (update_vec / update_scalar), the all-gather of a scalar weight, and
+// the host side of the launchers (argument check, SM count, world-size and
+// solver dispatch).  Every kernel
 // uses these except in the few places listed in DESIGN.md §3, where the helper
 // changed the kernel's spills or static instruction counts.
 #ifndef COS_SYNC_DEVICE_CUH_
@@ -419,6 +421,138 @@ __device__ __forceinline__ float sgd_scalar(const SyncParams& p, SegCursor c, ui
   return w;
 }
 
+// ------------------------------------------------ the other solvers' element
+
+// Regularize (as sgd_element_t), then ComputeUpdateValue of solver S, then Blob::Update w = (-1*g) + w, for one
+// element.  The CPU branch of each solver, one rounding per operation in the BLAS order of mkl_alternate.hpp
+// (axpby(a,x,b,y): y = b*y then y = a*x + y; add_scalar: y = y + d; scale: y = a*x; powx(x, 2) = x*x, powx(x, 0.5)
+// taken as the correctly rounded square root, DESIGN.md §7):
+//   Nesterov (nesterov_solver.cpp:21-41):  u = h; h = m*h; h = lr*g + h; u = (-m)*u; u = (1+m)*h + u; g = u
+//   AdaGrad  (adagrad_solver.cpp:21-50):   u = g*g; h = u + h; u = sqrt(h); u = u + d; u = g / u;
+//                                          g = 0*g; g = lr*u + g
+//   RMSProp  (rmsprop_solver.cpp:24-51):   u = g*g; h = rho*h; h = (1-rho)*u + h; then as AdaGrad from u = sqrt(h)
+//   AdaDelta (adadelta_solver.cpp:34-89):  u = g*g; h = m*h; h = (1-m)*u + h; u = d + h2; t = d + h; u = u / t;
+//                                          u = sqrt(u); g = g*u; u = g*g; h2 = m*h2; h2 = (1-m)*u + h2; g = lr*g
+// p.momentum is rho for RMSProp.  h2 is only read and written by AdaDelta.
+template <int S, bool L1>
+__device__ __forceinline__ void solver_element_t(const SyncParams& p, float g, float& w, float& h, float& h2, float lr,
+                                                 float ld) {
+  if (ld != 0.f) {
+    const float x = L1 ? static_cast<float>((0.f < w) - (w < 0.f)) : w;
+    g = __fadd_rn(__fmul_rn(ld, x), g);
+  }
+  if constexpr (S == kSolverNesterov) {
+    float u = h;
+    h = __fmul_rn(p.momentum, h);
+    h = __fadd_rn(__fmul_rn(lr, g), h);
+    u = __fmul_rn(p.neg_m, u);
+    u = __fadd_rn(__fmul_rn(p.one_plus_m, h), u);
+    g = u;
+  } else if constexpr (S == kSolverAdaGrad || S == kSolverRMSProp) {
+    float u = __fmul_rn(g, g);
+    if constexpr (S == kSolverAdaGrad) {
+      h = __fadd_rn(u, h);
+    } else {
+      h = __fmul_rn(p.momentum, h);
+      h = __fadd_rn(__fmul_rn(p.one_minus, u), h);
+    }
+    u = __fsqrt_rn(h);
+    u = __fadd_rn(u, p.delta);
+    u = __fdiv_rn(g, u);
+    g = __fmul_rn(0.f, g);
+    g = __fadd_rn(__fmul_rn(lr, u), g);
+  } else if constexpr (S == kSolverAdaDelta) {
+    float u = __fmul_rn(g, g);
+    h = __fmul_rn(p.momentum, h);
+    h = __fadd_rn(__fmul_rn(p.one_minus, u), h);
+    u = __fadd_rn(p.delta, h2);
+    const float t = __fadd_rn(p.delta, h);
+    u = __fdiv_rn(u, t);
+    u = __fsqrt_rn(u);
+    g = __fmul_rn(g, u);
+    u = __fmul_rn(g, g);
+    h2 = __fmul_rn(p.momentum, h2);
+    h2 = __fadd_rn(__fmul_rn(p.one_minus, u), h2);
+    g = __fmul_rn(lr, g);
+  }
+  w = __fadd_rn(__fmul_rn(-1.0f, g), w);
+}
+
+template <int S>
+__device__ __forceinline__ void solver_element(const SyncParams& p, float g, float& w, float& h, float& h2, float lr,
+                                               float ld) {
+  if (p.l1) solver_element_t<S, true>(p, g, w, h, h2, lr, ld);
+  else solver_element_t<S, false>(p, g, w, h, h2, lr, ld);
+}
+
+// sgd_vec for solver S != SGD: same blob-boundary split; AdaDelta reads and writes h2 at p.hist2 + i here
+template <int S>
+__device__ __forceinline__ void solver_vec(const SyncParams& p, SegCursor& c, uint64_t i, const float4& g, float4& w,
+                                           float4& h) {
+  float4 h2 = make_float4(0.f, 0.f, 0.f, 0.f);
+  if constexpr (S == kSolverAdaDelta) h2 = *reinterpret_cast<const float4*>(p.hist2 + i);
+  c.advance(i);
+  if (i + 3 < c.end[c.k]) {
+    const float lr = __fmul_rn(p.rate, c.lr_mult[c.k]);
+    const float ld = __fmul_rn(p.weight_decay, c.decay_mult[c.k]);
+    if (p.l1) {
+      solver_element_t<S, true>(p, g.x, w.x, h.x, h2.x, lr, ld);
+      solver_element_t<S, true>(p, g.y, w.y, h.y, h2.y, lr, ld);
+      solver_element_t<S, true>(p, g.z, w.z, h.z, h2.z, lr, ld);
+      solver_element_t<S, true>(p, g.w, w.w, h.w, h2.w, lr, ld);
+    } else {
+      solver_element_t<S, false>(p, g.x, w.x, h.x, h2.x, lr, ld);
+      solver_element_t<S, false>(p, g.y, w.y, h.y, h2.y, lr, ld);
+      solver_element_t<S, false>(p, g.z, w.z, h.z, h2.z, lr, ld);
+      solver_element_t<S, false>(p, g.w, w.w, h.w, h2.w, lr, ld);
+    }
+  } else {  // the vector straddles one or more blob boundaries
+    const float gg[4] = {g.x, g.y, g.z, g.w};
+    float ww[4] = {w.x, w.y, w.z, w.w};
+    float hh[4] = {h.x, h.y, h.z, h.w};
+    float h2h[4] = {h2.x, h2.y, h2.z, h2.w};
+    int k = c.k;
+#pragma unroll
+    for (int e = 0; e < 4; ++e) {
+      while (k < c.nseg - 1 && i + e >= c.end[k]) ++k;
+      solver_element<S>(p, gg[e], ww[e], hh[e], h2h[e], __fmul_rn(p.rate, c.lr_mult[k]),
+                        __fmul_rn(p.weight_decay, c.decay_mult[k]));
+    }
+    w = make_float4(ww[0], ww[1], ww[2], ww[3]);
+    h = make_float4(hh[0], hh[1], hh[2], hh[3]);
+    h2 = make_float4(h2h[0], h2h[1], h2h[2], h2h[3]);
+  }
+  if constexpr (S == kSolverAdaDelta) *reinterpret_cast<float4*>(p.hist2 + i) = h2;
+}
+
+template <int S>
+__device__ __forceinline__ float solver_scalar(const SyncParams& p, SegCursor c, uint64_t i, float g, float* wl,
+                                               float* hl) {
+  c.seek(i);
+  float w = wl[i], h = hl[i], h2 = 0.f;
+  if constexpr (S == kSolverAdaDelta) h2 = p.hist2[i];
+  solver_element<S>(p, g, w, h, h2, __fmul_rn(p.rate, c.lr_mult[c.k]), __fmul_rn(p.weight_decay, c.decay_mult[c.k]));
+  if constexpr (S == kSolverAdaDelta) p.hist2[i] = h2;
+  hl[i] = h;
+  wl[i] = w;
+  return w;
+}
+
+// What the kernels call: SGD goes through sgd_vec / sgd_scalar unchanged, so its instantiations compile as before.
+template <int S>
+__device__ __forceinline__ void update_vec(const SyncParams& p, SegCursor& c, uint64_t i, const float4& g, float4& w,
+                                           float4& h) {
+  if constexpr (S == kSolverSGD) sgd_vec(p, c, i, g, w, h);
+  else solver_vec<S>(p, c, i, g, w, h);
+}
+
+template <int S>
+__device__ __forceinline__ float update_scalar(const SyncParams& p, const SegCursor& c, uint64_t i, float g, float* wl,
+                                               float* hl) {
+  if constexpr (S == kSolverSGD) return sgd_scalar(p, c, i, g, wl, hl);
+  else return solver_scalar<S>(p, c, i, g, wl, hl);
+}
+
 // Scalar element i of shard s summed over every rank's diff_ (or bf16 wire) in the reference's order s, s+1, ...
 // (mod N), each term scaled by 1/N first: the scalar head / tail of the pull kernels, and every element when the
 // world size is known at run time only.
@@ -475,6 +609,19 @@ cudaError_t dispatch_world(int world, F&& f) {
     case 7: return f(std::integral_constant<int, 7>());
     case 8: return f(std::integral_constant<int, 8>());
     default: return f(std::integral_constant<int, 0>());
+  }
+}
+
+// f(std::integral_constant<int, S>()) with S = the SolverType p.solver; cudaErrorInvalidValue for any other value
+template <class F>
+cudaError_t dispatch_solver(int solver, F&& f) {
+  switch (solver) {
+    case kSolverSGD: return f(std::integral_constant<int, kSolverSGD>());
+    case kSolverNesterov: return f(std::integral_constant<int, kSolverNesterov>());
+    case kSolverAdaGrad: return f(std::integral_constant<int, kSolverAdaGrad>());
+    case kSolverRMSProp: return f(std::integral_constant<int, kSolverRMSProp>());
+    case kSolverAdaDelta: return f(std::integral_constant<int, kSolverAdaDelta>());
+    default: return cudaErrorInvalidValue;
   }
 }
 

@@ -78,6 +78,12 @@ typedef struct cos_solver_desc {
   int grad_dtype;              /* COS_GRAD_FP32 | COS_GRAD_BF16 */
   int init_iter;               /* iteration to resume from (0) */
   int regularization_l1;       /* SolverParameter.regularization_type: 0 = "L2" (default), 1 = "L1" */
+  /* SolverParameter.type: "SGD", "Nesterov", "AdaGrad", "RMSProp" or "AdaDelta"; NULL = "SGD".  Other types
+   * (Adam among them) fail at allocation, as do momentum != 0 with AdaGrad / RMSProp and rms_decay outside [0, 1)
+   * with RMSProp (the checks of the reference's solver constructors, sgd_solvers.hpp:70-100). */
+  const char* type;
+  float delta;                 /* SolverParameter.delta (AdaGrad, RMSProp, AdaDelta); Caffe's default is 1e-8 */
+  float rms_decay;             /* SolverParameter.rms_decay (RMSProp); Caffe's default is 0 */
 } cos_solver_desc;
 
 /* Gradient producer = Net::ForwardBackward of the reference (solver.cpp:221-223),
@@ -133,8 +139,8 @@ COS_API int cos_net_init(cos_net* net, int solver_index, int enable_nn);
 
 /* J:120 train / JN:383-413, CN:707-729: ONE Solver::Step (solver.cpp:194-273):
  * stage the input blobs host->device, run the gradient producer, then the
- * fused scale + reduce-scatter + SGD/momentum update + weight all-gather
- * kernel, ++iter.  data==NULL -> 0 with error "data is NULL" (JN:391-395). */
+ * fused scale + reduce-scatter + solver update (SGD, Nesterov, AdaGrad,
+ * RMSProp or AdaDelta) + weight all-gather kernel, ++iter.  data==NULL -> 0 with error "data is NULL" (JN:391-395). */
 COS_API int cos_net_train(cos_net* net, int solver_index, const cos_blob* data, int ndata);
 
 /* J:110 predict / JN:277-376: forward-only; not on the sync path -> always
@@ -183,6 +189,9 @@ COS_API int cos_net_set_forward_backward(cos_net* net, cos_forward_backward_fn f
 COS_API float* cos_net_data(cos_net* net, int solver_index);
 COS_API float* cos_net_diff(cos_net* net, int solver_index);
 COS_API float* cos_net_history(cos_net* net, int solver_index);
+/* AdaDelta's second history buffer (the history of updates, history_[n + i] of the reference), laid out like
+ * cos_net_history(); NULL for every other solver, which has no second buffer. */
+COS_API float* cos_net_update_history(cos_net* net, int solver_index);
 COS_API int64_t cos_net_param_count(cos_net* net);
 
 /* SocketSync::chunk (socket_sync_cpu.cpp:46-54): shard of `rank`. 1/0. */
@@ -197,8 +206,9 @@ COS_API float cos_net_last_loss(cos_net* net);
 /* THE HOT PATH.  Everything of Solver::Step after ForwardBackward plus the
  * next step's on_start, as one kernel launch on `cuda_stream` (NULL = the
  * net's own stream): diff *= 1/N, reduce-scatter over NVLink peer memory in
- * the reference's summation order, L2 decay, momentum SGD, w -= h, push of the
- * new weights to every peer, optional diff := 0 (ClearParamDiffs of the next
+ * the reference's summation order, L2 / L1 decay, the solver's update (SGD with
+ * momentum, Nesterov, AdaGrad, RMSProp or AdaDelta, in the operation order of
+ * the reference's CPU branch), w -= update, push of the new weights to every peer, optional diff := 0 (ClearParamDiffs of the next
  * Step), ++iter.  Asynchronous: returns after the launch.  Collective: every
  * rank must call it once per iteration. */
 COS_API int cos_net_sync_step(cos_net* net, int solver_index, void* cuda_stream);
@@ -215,7 +225,8 @@ COS_API int cos_net_synchronize(cos_net* net);
  * "grid" (CTAs, 0 = auto), "block" (threads, 0 = auto), "kernel" (-1 = auto,
  * 0 = LDG/STG pull kernel, 1 = TMA bulk-copy pull pipeline, 2 = push kernel
  * (stores only, bf16 cast in registers), 3 = NVLS multimem kernel, 4 = LL kernel
- * (flag-in-data words, no barrier / fence; small nets, cluster_size <= 8)),
+ * (flag-in-data words, no barrier / fence; small nets, cluster_size <= 8); kernels 1 and 3 run SGD only:
+ * with another solver a forced 1 runs kernel 0 and a forced 3 AUTO's choice),
  * "barrier_timeout_ms", "one_shot_max_bytes", "ll_max_bytes" / "push_max_bytes" /
  * "nvls_min_bytes" (AUTO thresholds on the message size 4P), "push_vecs" (push / LL
  * kernel grid sizing),
